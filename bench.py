@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          (N>1: launched by torch.distributed.run)
     python bench.py --impl reference ...                   (CPU restatement of the reference path)
+    python bench.py ... --dump-outputs DIR                 (also writes the placements of the last timed step)
 
 A "step" is one pass of the hot path over one batch of synthetic input: the 10 000-node snapshot is
 laid out on the device (gp_set_snapshot_device) and 100 000 pending applications are packed
@@ -192,6 +193,28 @@ def parity_word(results, gpu_driver, gpu_exec, gpu_off):
     return checked, mism
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, driver, executors, count):
+    """Writes the placements of one pack -- what a caller of gp_pack_batch receives -- as float64 .npy files:
+    driver_node [apps] and executor_nodes [sum(count)], the latter -1 for applications without a driver node (their
+    slots are undefined in the ABI, so they would differ from run to run).  Above DUMP_BYTES in all, executor_nodes is
+    a fixed, seeded sample of the slots and executor_nodes_index says which."""
+    os.makedirs(out_dir, exist_ok=True)
+    driver = np.asarray(driver, dtype=np.float64)
+    fits = np.repeat(driver >= 0, count)
+    arrays = {"driver_node": driver,
+              "executor_nodes": np.where(fits, np.asarray(executors[:len(fits)]), -1).astype(np.float64)}
+    room = DUMP_BYTES - driver.nbytes
+    if arrays["executor_nodes"].nbytes > room:
+        idx = np.sort(np.random.default_rng(0).choice(len(fits), room // 16, replace=False))
+        arrays["executor_nodes"] = arrays["executor_nodes"][idx]
+        arrays["executor_nodes_index"] = idx.astype(np.float64)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 def common_config(w: dict, q: int, world: int, total_exec: int) -> dict:
     """The `config` object -- identical in the repo arm and the reference arm (same workload, same sizes)."""
     return {"workload": w["desc"], "nodes": w["nodes"], "apps_per_gpu": q, "apps_total": q * world,
@@ -282,7 +305,11 @@ def main():
     ap.add_argument("--wire", default="compact", choices=["compact", "int64"],
                     help="host path layout: compact = what gp_pack_batch_wire allows for this batch; int64 = gp_pack_batch")
     ap.add_argument("--max-seconds", type=float, default=900.0, help="watchdog: abort if the run takes longer")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the placements of the last timed step (rank 0's block) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wd = _watchdog(args.max_seconds)
     w = WORKLOADS[args.workload]
 
@@ -294,8 +321,8 @@ def main():
     import torch
     import torch.distributed as dist
     import k8s_spark_scheduler_b200 as g
-    if not os.path.exists(g.native.LIB_PATH):      # normally prebuilt in-tree by __graft_entry__.build()
-        g.native.build()
+    if not os.path.exists(g.native.LIB_PATH):      # the benchmark never compiles into the tree it runs from
+        raise SystemExit(f"{g.native.LIB_PATH} is missing: build it first (python __graft_entry__.py)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -536,6 +563,8 @@ def main():
                 rd, _ = shm.block(r)
                 if int(rd.astype(np.int64).sum()) != int(sums[r][0].item()):
                     path_mism += 1
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dev_driver_np, dev_exec_np, a["count"])
 
     # ---- roofline of the dominant kernel (pack) ----------------------------------------------------
     peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")

@@ -39,7 +39,8 @@ def test_library_exports_every_declared_symbol(native):
 
 
 def test_library_contains_sm100a_code(native):
-    out = subprocess.check_output(["cuobjdump", "-lelf", native.LIB_PATH], text=True)
+    cuobjdump = os.path.join(os.path.dirname(native._nvcc()), "cuobjdump")   # the toolkit that built the library
+    out = subprocess.check_output([cuobjdump, "-lelf", native.LIB_PATH], text=True)
     assert "sm_100a" in out
 
 
