@@ -152,88 +152,176 @@ __device__ __forceinline__ int32_t find_group(const int32_t* off, int32_t n_grou
     return lo;
 }
 
-__global__ void gp_build_groups(int32_t n_groups, const int32_t* __restrict__ exec_off, const int32_t* __restrict__ drv_off,
-                                GroupDesc* __restrict__ groups) {
-    int32_t g = blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= n_groups) return;
-    GroupDesc d;
-    d.sbase = exec_off[g] + drv_off[g];
-    d.ne = exec_off[g + 1] - exec_off[g];
-    d.dbase = drv_off[g];
-    d.nd = drv_off[g + 1] - drv_off[g];
-    groups[g] = d;
-}
+// The slot layout is built by two kernels and nothing else (no memset, no copy node), so that a snapshot taken every
+// Predicate costs two launches:
+//   gp_snap_slots   executor slots, group descriptors, per-node inverse indices into both orders, and per-CTA partial
+//                   maxima (every slot that gets written holds the values of a node of one of the two orders, so the
+//                   snapshot-wide facts are a fold over both orders -- no need to know yet which driver takes a spare slot);
+//   gp_snap_finish  SnapMeta from the partials, driver slots (spare slots included), node_slot with one writer per node,
+//                   the compact view, and (gp_set_snapshot_device) the node-table copy.
+// The inverse indices are never reset: inv[v] is believed only if the order holds v at that position.
+// Both kernels bound the order lengths by exec_off[n_groups] / drv_off[n_groups]: gp_prepare_cluster passes upper bounds.
+constexpr int kSnapThreads = 256;
+constexpr int kSnapMaxParts = 256;          // grid bound of both kernels (grid-stride loops); partials gp_snap_finish folds
 
-// snapshot-wide facts: negative gpu availability, per-dimension maxima (bounds for the fast class)
-// Called by the threads of a warp that own a node (`active` = their mask): the warp combines its values with
-// shuffles and issues at most one atomic per dimension.
-__device__ __forceinline__ long long warp_max_ll(unsigned active, long long v) {
+struct SnapPart { long long v[4]; };        // max(cpu, 0), max(mem, 0), max(gpu, 0), any gpu < 0
+
+struct SnapLayout {
+    int32_t n_exec, n_drv, n_groups, n_nodes, n_slots;     // n_exec / n_drv may be upper bounds
+    const int32_t *exec_off, *drv_off, *exec_order, *drv_order;
+    const int64_t *cpu, *mem, *gpu;                         // node table; gpu may be NULL (= 0)
+    GroupDesc* groups;
+    longlong2* pair;
+    int64_t* sgpu;
+    uint2* pair32;
+    int32_t *slot_node, *node_slot, *drv_slot;
+    int32_t *inv_exec, *inv_drv;                            // [n_nodes] each
+    SnapPart* parts;                                        // [kSnapMaxParts]
+    SnapMeta* meta;
+    int64_t *copy_cpu, *copy_mem, *copy_gpu;                // node-table copy, or NULL
+    __device__ __forceinline__ int32_t ne_all() const { return min(n_exec, exec_off[n_groups]); }
+    __device__ __forceinline__ int32_t nd_all() const { return min(n_drv, drv_off[n_groups]); }
+    __device__ __forceinline__ int64_t gpu_of(int32_t v) const { return gpu ? gpu[v] : 0; }
+    __device__ __forceinline__ int32_t exec_slot(int32_t e) const {
+        const int32_t g = find_group(exec_off, n_groups, e);
+        return drv_off[g] + e;                              // exec_off[g] + drv_off[g] + (e - exec_off[g])
+    }
+    // position of node v in the executor order, or -1
+    __device__ __forceinline__ int32_t exec_pos(int32_t v, int32_t ne) const {
+        const int32_t e = inv_exec[v];
+        return (e >= 0 && e < ne && exec_order[e] == v) ? e : -1;
+    }
+    // driver candidate j whose node has global executor slot es (-1: none): it uses that slot when it lies in the
+    // driver's own group, else its spare slot ne + (j - dbase)
+    struct DrvSlot { int32_t sbase, local, spare; };        // group base, group-local slot, global spare slot
+    __device__ __forceinline__ DrvSlot driver_slot(int32_t j, int32_t es) const {
+        const int32_t g = find_group(drv_off, n_groups, j);
+        const int32_t sbase = exec_off[g] + drv_off[g], ne = exec_off[g + 1] - exec_off[g];
+        const int32_t spare = ne + (j - drv_off[g]);
+        return DrvSlot{sbase, (es >= sbase && es < sbase + ne) ? es - sbase : spare, sbase + spare};
+    }
+};
+
+// max over the block of four non-negative values; the result is returned to every thread
+__device__ __forceinline__ void block_max4(long long v[4]) {
+    __shared__ long long s_red[kSnapThreads / 32][4];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
 #pragma unroll
-    for (int d = 16; d >= 1; d >>= 1) {
-        long long o = __shfl_xor_sync(active, v, d);     // lanes outside `active` return their own value: harmless for max
-        v = o > v ? o : v;
-    }
-    return v;
-}
-__device__ __forceinline__ void note_node(SnapMeta* meta, int64_t cv, int64_t mv, int64_t gv) {
-    const unsigned active = __activemask();
-    const bool full = active == 0xffffffffu;
-    if (__any_sync(active, gv < 0) && (threadIdx.x & 31) == (__ffs(active) - 1)) atomicOr(&meta->flags, kSnapGpuNegative);
-    long long c = cv, m = mv, g = gv;
-    if (full) { c = warp_max_ll(active, c); m = warp_max_ll(active, m); g = warp_max_ll(active, g); }
-    if (!full || (threadIdx.x & 31) == 0) {
-        if (c > 0 && c > meta->max_avail[0]) atomicMax(&meta->max_avail[0], c);
-        if (m > 0 && m > meta->max_avail[1]) atomicMax(&meta->max_avail[1], m);
-        if (g > 0 && g > meta->max_avail[2]) atomicMax(&meta->max_avail[2], g);
+    for (int k = 0; k < 4; ++k)
+#pragma unroll
+        for (int d = 16; d >= 1; d >>= 1) v[k] = max(v[k], __shfl_xor_sync(kFull, v[k], d));
+    if (lane == 0)
+#pragma unroll
+        for (int k = 0; k < 4; ++k) s_red[w][k] = v[k];
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        long long m = 0;
+        for (int t = 0; t < kSnapThreads / 32; ++t) m = max(m, s_red[t][k]);
+        v[k] = m;
     }
 }
 
-// executor-order entries -> slots [sbase, sbase+ne)
-__global__ void gp_build_exec_slots(int32_t n_exec, int32_t n_groups,
-                                    const int32_t* __restrict__ exec_off, const int32_t* __restrict__ drv_off,
-                                    const int32_t* __restrict__ exec_order,
-                                    const int64_t* __restrict__ cpu, const int64_t* __restrict__ mem, const int64_t* __restrict__ gpu,
-                                    longlong2* __restrict__ pair, int64_t* __restrict__ sgpu, int32_t* __restrict__ slot_node,
-                                    int32_t* __restrict__ node_slot, SnapMeta* __restrict__ meta) {
-    int32_t e = blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n_exec || e >= exec_off[n_groups]) return;     // n_exec may be an upper bound (device-built orders)
-    int32_t g = find_group(exec_off, n_groups, e);
-    int32_t slot = exec_off[g] + drv_off[g] + (e - exec_off[g]);
-    int32_t node = exec_order[e];
-    const int64_t cv = cpu[node], mv = mem[node], gv = gpu ? gpu[node] : 0;
-    pair[slot] = make_longlong2(cv, mv);
-    sgpu[slot] = gv;
-    note_node(meta, cv, mv, gv);
-    slot_node[slot] = node;
-    node_slot[node] = slot;
+__device__ __forceinline__ void fold_node(long long v[4], int64_t cv, int64_t mv, int64_t gv) {
+    v[0] = max(v[0], (long long)cv); v[1] = max(v[1], (long long)mv); v[2] = max(v[2], (long long)gv);
+    if (gv < 0) v[3] = 1;
 }
 
-// driver-order entries -> group-local slot (an executor slot, or the spare slot ne + j)
-__global__ void gp_build_driver_slots(int32_t n_drv, int32_t n_groups,
-                                      const int32_t* __restrict__ exec_off, const int32_t* __restrict__ drv_off,
-                                      const int32_t* __restrict__ drv_order,
-                                      const int64_t* __restrict__ cpu, const int64_t* __restrict__ mem, const int64_t* __restrict__ gpu,
-                                      longlong2* __restrict__ pair, int64_t* __restrict__ sgpu, int32_t* __restrict__ slot_node,
-                                      int32_t* __restrict__ node_slot, int32_t* __restrict__ drv_slot, SnapMeta* __restrict__ meta) {
-    int32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n_drv || j >= drv_off[n_groups]) return;       // n_drv may be an upper bound
-    int32_t g = find_group(drv_off, n_groups, j);
-    int32_t sbase = exec_off[g] + drv_off[g];
-    int32_t ne = exec_off[g + 1] - exec_off[g];
-    int32_t node = drv_order[j];
-    int32_t ns = node_slot[node];
-    if (ns >= sbase && ns < sbase + ne) {
-        drv_slot[j] = ns - sbase;
-    } else {
-        int32_t local = ne + (j - drv_off[g]);
-        int32_t slot = sbase + local;
-        const int64_t cv = cpu[node], mv = mem[node], gv = gpu ? gpu[node] : 0;
-        pair[slot] = make_longlong2(cv, mv);
-        sgpu[slot] = gv;
-        note_node(meta, cv, mv, gv);
-        slot_node[slot] = node;
-        node_slot[node] = slot;          // the node's availability lives in its spare slot (gp_reserve_placements / gp_apply_usage_delta)
-        drv_slot[j] = local;
+__global__ void __launch_bounds__(kSnapThreads) gp_snap_slots(SnapLayout L) {
+    const int32_t ne = L.ne_all(), nd = L.nd_all();
+    const int32_t n = max(max(ne, nd), L.n_groups);
+    long long acc[4] = {0, 0, 0, 0};
+    for (int32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < n; t += gridDim.x * blockDim.x) {
+        if (t < L.n_groups) {
+            GroupDesc d;
+            d.sbase = L.exec_off[t] + L.drv_off[t];
+            d.ne = L.exec_off[t + 1] - L.exec_off[t];
+            d.dbase = L.drv_off[t];
+            d.nd = L.drv_off[t + 1] - L.drv_off[t];
+            L.groups[t] = d;
+        }
+        if (t < ne) {             // executor-order entry t -> slot sbase + (t - exec_off[g])
+            const int32_t slot = L.exec_slot(t);
+            const int32_t v = L.exec_order[t];
+            const int64_t cv = L.cpu[v], mv = L.mem[v], gv = L.gpu_of(v);
+            L.pair[slot] = make_longlong2(cv, mv);
+            L.sgpu[slot] = gv;
+            L.slot_node[slot] = v;
+            L.inv_exec[v] = t;
+            fold_node(acc, cv, mv, gv);
+        }
+        if (t < nd) {             // driver-order entry: its slot is decided in gp_snap_finish
+            const int32_t v = L.drv_order[t];
+            L.inv_drv[v] = t;
+            fold_node(acc, L.cpu[v], L.mem[v], L.gpu_of(v));
+        }
+    }
+    block_max4(acc);
+    if (threadIdx.x == 0) L.parts[blockIdx.x] = SnapPart{{acc[0], acc[1], acc[2], acc[3]}};
+}
+
+// compact view, 8 bytes per slot instead of 16 (negative availability -> 0: capacity 0 either way).  Its shifts are the
+// smallest S with max_avail >> S < 2^32.
+__device__ __forceinline__ int shift_for(long long mx) {
+    if (mx <= 0) return 0;
+    const int bits = 64 - __clzll(mx);
+    return bits > 32 ? bits - 32 : 0;
+}
+__device__ __forceinline__ uint2 compact_pair(longlong2 v, int s0, int s1) {
+    return make_uint2(v.x < 0 ? 0u : (uint32_t)((unsigned long long)v.x >> s0), v.y < 0 ? 0u : (uint32_t)((unsigned long long)v.y >> s1));
+}
+
+__global__ void __launch_bounds__(kSnapThreads) gp_snap_finish(SnapLayout L, int32_t n_parts) {
+    long long acc[4] = {0, 0, 0, 0};
+    for (int p = threadIdx.x; p < n_parts; p += blockDim.x)
+#pragma unroll
+        for (int k = 0; k < 4; ++k) acc[k] = max(acc[k], L.parts[p].v[k]);
+    block_max4(acc);
+    const int s0 = shift_for(acc[0]), s1 = shift_for(acc[1]);
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        SnapMeta m{};
+        m.flags = acc[3] ? kSnapGpuNegative : 0;
+        m.max_avail[0] = acc[0]; m.max_avail[1] = acc[1]; m.max_avail[2] = acc[2];
+        m.shift32[0] = s0; m.shift32[1] = s1;
+        *L.meta = m;
+    }
+    const int32_t ne = L.ne_all(), nd = L.nd_all();
+    const int32_t used = min(L.exec_off[L.n_groups] + L.drv_off[L.n_groups], L.n_slots);
+    const int32_t n = max(max(ne, nd), max(L.n_slots, L.n_nodes) + 1);
+    for (int32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < n; t += gridDim.x * blockDim.x) {
+        if (t < nd) {             // driver candidate t: its executor slot, or its spare slot holding the node's values
+            const int32_t v = L.drv_order[t];
+            const int32_t e = L.exec_pos(v, ne);
+            const SnapLayout::DrvSlot d = L.driver_slot(t, e >= 0 ? L.exec_slot(e) : -1);
+            L.drv_slot[t] = d.local;
+            if (d.sbase + d.local == d.spare) {
+                const longlong2 pv = make_longlong2(L.cpu[v], L.mem[v]);
+                L.pair[d.spare] = pv;
+                L.sgpu[d.spare] = L.gpu_of(v);
+                L.pair32[d.spare] = compact_pair(pv, s0, s1);
+                L.slot_node[d.spare] = v;
+            } else {
+                L.slot_node[d.spare] = -1;              // unused spare slot
+            }
+        }
+        if (t < ne) {
+            const int32_t slot = L.exec_slot(t);
+            L.pair32[slot] = compact_pair(L.pair[slot], s0, s1);
+        }
+        if (t >= used && t <= L.n_slots) L.slot_node[t] = -1;
+        if (t < L.n_nodes) {      // one writer per node: its spare slot if it has one, else its executor slot, else -1
+            const int32_t e = L.exec_pos(t, ne);
+            int32_t slot = e >= 0 ? L.exec_slot(e) : -1;
+            const int32_t j = L.inv_drv[t];
+            if (j >= 0 && j < nd && L.drv_order[j] == t) {
+                const SnapLayout::DrvSlot d = L.driver_slot(j, slot);
+                slot = d.sbase + d.local;
+            }
+            L.node_slot[t] = slot;
+            if (L.copy_cpu) { L.copy_cpu[t] = L.cpu[t]; L.copy_mem[t] = L.mem[t]; L.copy_gpu[t] = L.gpu_of(t); }
+        } else if (t == L.n_nodes) {
+            L.node_slot[t] = -1;
+        }
     }
 }
 
@@ -252,25 +340,14 @@ __global__ void gp_multi_copy(CopyJobs jobs) {
     }
 }
 
-// After the slots are laid out: the compact view, 8 bytes per slot instead of 16 (negative availability -> 0:
-// capacity 0 either way).  Its shifts are the smallest S with max_avail >> S < 2^32; every thread derives them
-// from SnapMeta::max_avail, thread 0 publishes them for gp_prep_apps.
-__device__ __forceinline__ int shift_for(long long mx) {
-    if (mx <= 0) return 0;
-    const int bits = 64 - __clzll(mx);
-    return bits > 32 ? bits - 32 : 0;
-}
+// the compact view again after `pair` changed in place (FIFO packing, availability upkeep); thread 0 publishes the shifts
 __global__ void gp_fill_pair32(int32_t n_slots, const longlong2* __restrict__ pair, SnapMeta* __restrict__ meta,
                                uint2* __restrict__ pair32) {
     const int s0 = shift_for(meta->max_avail[0]), s1 = shift_for(meta->max_avail[1]);
     const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0) { meta->shift32[0] = s0; meta->shift32[1] = s1; }
     if (i >= n_slots) return;
-    const longlong2 v = pair[i];
-    uint2 o;
-    o.x = v.x < 0 ? 0u : (uint32_t)((unsigned long long)v.x >> s0);
-    o.y = v.y < 0 ? 0u : (uint32_t)((unsigned long long)v.y >> s1);
-    pair32[i] = o;
+    pair32[i] = compact_pair(pair[i], s0, s1);
 }
 
 // slots -> node-table order (gp_get_snapshot)
@@ -340,6 +417,7 @@ struct gp_ctx {
     DevBuf node_cpu, node_mem, node_gpu;        // node-table order (as given)
     DevBuf exec_off, drv_off, exec_order, drv_order;
     DevBuf pair, pair32, sgpu, slot_node, node_slot, drv_slot, groups, snap_flags;
+    DevBuf snap_aux;                              // slot layout scratch (build_snapshot_device)
 
     // batch staging
     DevBuf a_dcpu, a_dmem, a_dgpu, a_ecpu, a_emem, a_egpu, a_count, a_group, a_skip, a_off;
@@ -360,8 +438,8 @@ struct gp_ctx {
     int pack_ctas_per_sm[3] = {0, 0, 0};            // occupancy of gp_pack_independent<ALGO> on this device
     int tab_ctas_per_sm[2][2] = {{0, 0}, {0, 0}};   // occupancy of gp_pack_tables<ALGO, OUT>
     bool tab_attr_set[2] = {false, false};
-    // per pipeline lane: shape hash + header, capacity tables, group totals, per-application shape slot
-    struct TableSet { DevBuf hdr, table, total, app_slot; } tabs[kLanes];
+    // per pipeline lane: shape hash + header, capacity tables, group totals, expansion lists, per-application shape slot
+    struct TableSet { DevBuf hdr, table, total, expand, app_slot; } tabs[kLanes];
     bool record_events = true;                    // CUDA events around the kernels (gp_last_stats); the pipelined host path skips them
     int use_graphs = 1;                           // GANGPACK_GRAPHS=0: always issue the launches one by one
     GraphCache g_chunk[kMaxChunks + 1];           // per pipelined chunk (+1: an unchunked batch on the context's own stream): classify .. scan
@@ -536,12 +614,12 @@ void gp_destroy(gp_ctx* c) {
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
     DevBuf* bufs[] = {&c->node_cpu, &c->node_mem, &c->node_gpu, &c->exec_off, &c->drv_off, &c->exec_order, &c->drv_order,
-                      &c->pair, &c->pair32, &c->sgpu, &c->slot_node, &c->node_slot, &c->drv_slot, &c->groups, &c->snap_flags,
+                      &c->pair, &c->pair32, &c->sgpu, &c->slot_node, &c->node_slot, &c->drv_slot, &c->groups, &c->snap_flags, &c->snap_aux,
                       &c->a_dcpu, &c->a_dmem, &c->a_dgpu, &c->a_ecpu, &c->a_emem, &c->a_egpu, &c->a_count, &c->a_group,
                       &c->a_skip, &c->a_off, &c->prep, &c->r_driver, &c->r_exec, &c->scratch, &c->dev_misc, &c->gmin, &c->sortbuf, &c->usagebuf, &c->reschedbuf,
                       &c->off_dev, &c->fifo_list, &c->sched, &c->zonebuf};
     for (DevBuf* b : bufs) b->release();
-    for (auto& t : c->tabs) { t.hdr.release(); t.table.release(); t.total.release(); t.app_slot.release(); }
+    for (auto& t : c->tabs) { t.hdr.release(); t.table.release(); t.total.release(); t.expand.release(); t.app_slot.release(); }
     for (auto& g : c->g_chunk) g.reset();
     c->g_snapshot.reset();
     if (c->pinned_misc) cudaFreeHost(c->pinned_misc);
@@ -599,8 +677,10 @@ gp_status gp_synchronize(gp_ctx* ctx) {
 
 // ---- snapshot ---------------------------------------------------------------------------------
 
-// Build the slot layout from DEVICE-resident gp_nodes arrays on `st`.
-static gp_status build_snapshot_device(gp_ctx* c, const gp_nodes* dn, int32_t n_exec, int32_t n_drv, cudaStream_t st) {
+// Build the slot layout from DEVICE-resident gp_nodes arrays on `st` (gp_snap_slots + gp_snap_finish).  copy_nodes: the
+// second kernel also copies the node table into node_cpu/mem/gpu (gp_set_snapshot_device; gp_set_snapshot has it there).
+static gp_status build_snapshot_device(gp_ctx* c, const gp_nodes* dn, int32_t n_exec, int32_t n_drv, cudaStream_t st,
+                                       bool copy_nodes = false) {
     const int32_t n_slots = n_exec + n_drv;
     GP_CUDA(c, c->pair.reserve(sizeof(longlong2) * (size_t)(n_slots + 1)));
     GP_CUDA(c, c->pair32.reserve(sizeof(uint2) * (size_t)(n_slots + 1)));
@@ -609,27 +689,27 @@ static gp_status build_snapshot_device(gp_ctx* c, const gp_nodes* dn, int32_t n_
     GP_CUDA(c, c->node_slot.reserve(sizeof(int32_t) * (size_t)(dn->n_nodes + 1)));
     GP_CUDA(c, c->drv_slot.reserve(sizeof(int32_t) * (size_t)(n_drv + 1)));
     GP_CUDA(c, c->groups.reserve(sizeof(GroupDesc) * (size_t)dn->n_groups));
-    struct { gp_nodes dn; int32_t n_exec, n_drv; void* buf[8]; } key{};
-    key.dn = *dn; key.n_exec = n_exec; key.n_drv = n_drv;
-    void* bufs[8] = {c->pair.p, c->pair32.p, c->sgpu.p, c->slot_node.p, c->node_slot.p, c->drv_slot.p, c->groups.p, c->snap_flags.p};
-    std::memcpy(key.buf, bufs, sizeof(bufs));
-    gp_status rs = run_cached(c, c->g_snapshot, &key, sizeof(key), st, [&](int& launches) -> gp_status {
-        GP_CUDA(c, cudaMemsetAsync(c->slot_node.p, 0xFF, sizeof(int32_t) * (size_t)(n_slots + 1), st));
-        GP_CUDA(c, cudaMemsetAsync(c->node_slot.p, 0xFF, sizeof(int32_t) * (size_t)(dn->n_nodes + 1), st));
-        GP_CUDA(c, cudaMemsetAsync(c->snap_flags.p, 0, sizeof(SnapMeta), st));
-        const int T = 256;
-        gp_build_groups<<<(dn->n_groups + T - 1) / T, T, 0, st>>>(dn->n_groups, dn->exec_off, dn->drv_off, c->groups.as<GroupDesc>());
-        if (n_exec > 0)
-            gp_build_exec_slots<<<(n_exec + T - 1) / T, T, 0, st>>>(
-                n_exec, dn->n_groups, dn->exec_off, dn->drv_off, dn->exec_order, dn->avail_cpu_milli, dn->avail_mem_bytes,
-                dn->avail_gpu, c->pair.as<longlong2>(), c->sgpu.as<int64_t>(), c->slot_node.as<int32_t>(),
-                c->node_slot.as<int32_t>(), c->snap_flags.as<SnapMeta>());
-        if (n_drv > 0)
-            gp_build_driver_slots<<<(n_drv + T - 1) / T, T, 0, st>>>(
-                n_drv, dn->n_groups, dn->exec_off, dn->drv_off, dn->drv_order, dn->avail_cpu_milli, dn->avail_mem_bytes,
-                dn->avail_gpu, c->pair.as<longlong2>(), c->sgpu.as<int64_t>(), c->slot_node.as<int32_t>(),
-                c->node_slot.as<int32_t>(), c->drv_slot.as<int32_t>(), c->snap_flags.as<SnapMeta>());
-        gp_fill_pair32<<<(n_slots + T) / T, T, 0, st>>>(n_slots, c->pair.as<longlong2>(), c->snap_flags.as<SnapMeta>(), c->pair32.as<uint2>());
+    // [per-CTA partials | inverse executor-order index | inverse driver-order index]
+    GP_CUDA(c, c->snap_aux.reserve(sizeof(SnapPart) * (size_t)kSnapMaxParts + 2 * sizeof(int32_t) * (size_t)(dn->n_nodes + 1)));
+    SnapLayout L;
+    std::memset(&L, 0, sizeof(L));      // the record is also the graph key: no indeterminate padding
+    L.n_exec = n_exec; L.n_drv = n_drv; L.n_groups = dn->n_groups; L.n_nodes = dn->n_nodes; L.n_slots = n_slots;
+    L.exec_off = dn->exec_off; L.drv_off = dn->drv_off; L.exec_order = dn->exec_order; L.drv_order = dn->drv_order;
+    L.cpu = dn->avail_cpu_milli; L.mem = dn->avail_mem_bytes; L.gpu = dn->avail_gpu;
+    L.groups = c->groups.as<GroupDesc>(); L.pair = c->pair.as<longlong2>(); L.sgpu = c->sgpu.as<int64_t>();
+    L.pair32 = c->pair32.as<uint2>(); L.slot_node = c->slot_node.as<int32_t>(); L.node_slot = c->node_slot.as<int32_t>();
+    L.drv_slot = c->drv_slot.as<int32_t>(); L.meta = c->snap_flags.as<SnapMeta>();
+    L.parts = c->snap_aux.as<SnapPart>();
+    L.inv_exec = reinterpret_cast<int32_t*>(L.parts + kSnapMaxParts);
+    L.inv_drv = L.inv_exec + (dn->n_nodes + 1);
+    if (copy_nodes) { L.copy_cpu = c->node_cpu.as<int64_t>(); L.copy_mem = c->node_mem.as<int64_t>(); L.copy_gpu = c->node_gpu.as<int64_t>(); }
+    auto grid = [](int64_t work) { return (int)std::max<int64_t>(1, std::min<int64_t>((work + kSnapThreads - 1) / kSnapThreads, kSnapMaxParts)); };
+    const int g1 = grid(std::max<int64_t>(std::max(n_exec, n_drv), dn->n_groups));
+    const int g2 = grid(std::max<int64_t>(std::max(n_exec, n_drv), (int64_t)std::max(n_slots, dn->n_nodes) + 1));
+    // every argument of both launches: the layout record and the two grid sizes (which follow from it)
+    gp_status rs = run_cached(c, c->g_snapshot, &L, sizeof(L), st, [&](int& launches) -> gp_status {
+        gp_snap_slots<<<g1, kSnapThreads, 0, st>>>(L);
+        gp_snap_finish<<<g2, kSnapThreads, 0, st>>>(L, g1);
         GP_CUDA(c, cudaGetLastError());
         launches = 0;       // (the snapshot layout is not part of a pack call's launch count)
         return GP_OK;
@@ -752,16 +832,10 @@ gp_status gp_set_snapshot_device(gp_ctx* c, const gp_nodes* dn, int32_t n_exec, 
         return fail(c, GP_ERR_INVALID, "gp_set_snapshot_device: missing arrays or bad sizes");
     GP_CUDA(c, cudaSetDevice(c->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
-    // keep a node-table copy so gp_get_snapshot can answer for nodes outside every group
-    const size_t nb = sizeof(int64_t) * (size_t)(dn->n_nodes + 1), vb = sizeof(int64_t) * (size_t)dn->n_nodes;
+    // keep a node-table copy so gp_get_snapshot can answer for nodes outside every group (written by gp_snap_finish)
+    const size_t nb = sizeof(int64_t) * (size_t)(dn->n_nodes + 1);
     GP_CUDA(c, c->node_cpu.reserve(nb)); GP_CUDA(c, c->node_mem.reserve(nb)); GP_CUDA(c, c->node_gpu.reserve(nb));
-    if (vb) {
-        GP_CUDA(c, cudaMemcpyAsync(c->node_cpu.p, dn->avail_cpu_milli, vb, cudaMemcpyDeviceToDevice, st));
-        GP_CUDA(c, cudaMemcpyAsync(c->node_mem.p, dn->avail_mem_bytes, vb, cudaMemcpyDeviceToDevice, st));
-        if (dn->avail_gpu) GP_CUDA(c, cudaMemcpyAsync(c->node_gpu.p, dn->avail_gpu, vb, cudaMemcpyDeviceToDevice, st));
-        else GP_CUDA(c, cudaMemsetAsync(c->node_gpu.p, 0, vb, st));
-    }
-    return build_snapshot_device(c, dn, n_exec, n_drv, st);
+    return build_snapshot_device(c, dn, n_exec, n_drv, st, true);
 }
 
 gp_status gp_get_snapshot(gp_ctx* c, int64_t* cpu, int64_t* mem, int64_t* gpu) {
@@ -916,6 +990,7 @@ static gp_status pack_device_range(gp_ctx* c, const DevApps& da, int32_t lo, int
         if (use_tables) {
             GP_CUDA(c, T.table.reserve(sizeof(uint32_t) * (size_t)kMaxShapes * (size_t)((c->n_slots + 4) & ~3)));
             GP_CUDA(c, T.total.reserve(3 * sizeof(uint32_t) * (size_t)kMaxShapes * (size_t)c->n_groups));   // total | firstfit | first_host
+            GP_CUDA(c, T.expand.reserve(sizeof(int32_t) * (size_t)kMaxShapes * (size_t)c->n_groups * kExpandCap));
         }
         ShapeTables tabs;
         tabs.hdr = T.hdr.as<ShapeHeader>();
@@ -924,6 +999,7 @@ static gp_status pack_device_range(gp_ctx* c, const DevApps& da, int32_t lo, int
         tabs.table = T.table.as<uint32_t>(); tabs.total = T.total.as<uint32_t>();
         tabs.firstfit = reinterpret_cast<int32_t*>(T.total.as<uint32_t>() + (size_t)kMaxShapes * (size_t)c->n_groups);
         tabs.first_host = tabs.firstfit + (size_t)kMaxShapes * (size_t)c->n_groups;
+        tabs.expand = T.expand.as<int32_t>();
         tabs.pitch = (c->n_slots + 4) & ~3; tabs.n_groups = c->n_groups;      // rows start 16-byte aligned
         int64_t* off_out = nullptr;
         if (!da.cols.off) {                       // derive the offsets on the device

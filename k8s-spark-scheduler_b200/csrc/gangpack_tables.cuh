@@ -19,15 +19,17 @@
 //                         thread evaluates 4 consecutive nodes, a block-wide exclusive scan turns capacities into the
 //                         prefix table  S[i] = sum_{n<i} min(cap(n|0), CLAMP)   (tightly-pack) or
 //                                       M[i] = #{n<i : cap(n|0) >= 1}            (distribute-evenly);
+//                         and, from the same tile, the expansion list E (node n repeated c(n) times, cut at kExpandCap);
 //       (same launch, second half of the grid: one CTA per (driver shape, instance group) finds the first driver candidate
 //       the shape fits on);
 //   K3 gp_decide_tables   ONE THREAD per application (with the tables a decision is O(log N + k) scalar work -- a warp per
 //                         application, right for an O(N) scan, would idle 31 lanes): feasibility is
 //                         S[ne] - delta(d) >= k  per driver candidate d starting at the shape's first fit (delta = what the
 //                         driver displaces on its own node: O(1) per candidate, the reference's loop binpack.go:67-85
-//                         verbatim), the walk starts at the shape's first hosting node (one word per (shape, group), written
-//                         by K2), ExecutorNodes is emitted by walking the table from there with the next word always in
-//                         flight (zero-capacity runs are jumped by a galloping search).
+//                         verbatim); ExecutorNodes is a prefix of E with the driver's node spliced in, copied by the whole
+//                         warp (32 entries per step); placements longer than E walk the table from the shape's first
+//                         hosting node (one word per (shape, group), written by K2) with the next word always in flight
+//                         (zero-capacity runs are jumped by a galloping search).
 // What the tables cannot answer exactly -- more than kMaxShapes distinct shapes in a batch, executor counts above the table
 // clamp, distribute-evenly placements that need more than one round -- is appended, already prepared (PrepApp), to a list
 // that the warp-per-application scan kernel gp_pack_listed (the node-order scan of gangpack_kernels.cuh) works off.
@@ -45,6 +47,11 @@ constexpr int kMaxShapes = 64;        // dense tables per batch
 constexpr int kTabThreads = 1024;
 constexpr int kTabPerThread = 4;
 constexpr int kTabTile = kTabThreads * kTabPerThread;     // 4096 nodes per tile: 64 KB of (cpu, mem)
+// Entries of the expansion list of one (shape, instance group): the node-major expansion E of the shape's capacities
+// (node n repeated c(n) times, E[S[n] .. S[n+1]) = n), cut at kExpandCap.  The placement of every application of the
+// shape that needs at most kExpandCap entries (k executors plus what its driver displaces) is copied from it; longer
+// ones walk the prefix table.  The bench.py workloads place at most 128 executors per application.
+constexpr int kExpandCap = 1024;
 
 struct __align__(16) ShapeEntry {     // 96 bytes
     unsigned long long key;           // fingerprint, never 0; 0 = empty (claimed with atomicCAS)
@@ -82,6 +89,7 @@ struct ShapeTables {
     uint32_t* total;                  // [kMaxShapes][n_groups]
     int32_t* firstfit;                // [kMaxShapes][n_groups] first driver-order position the driver shape fits on (nd: none)
     int32_t* first_host;              // [kMaxShapes][n_groups] first executor-order position with capacity > 0 for the shape (ne: none)
+    int32_t* expand;                  // [kMaxShapes][n_groups][kExpandCap] expansion list: entry t is the node that hosts executor t
     int32_t pitch;                    // row length (>= n_slots, multiple of 4)
     int32_t n_groups;
 };
@@ -277,6 +285,7 @@ __global__ void __launch_bounds__(kTabThreads, 1) gp_build_shape_tables(Snapshot
     const longlong2* gpair = s.pair + g.sbase;
     const int64_t* ggpu = s.gpu + g.sbase;
     uint32_t* out = tabs.table + (size_t)id * tabs.pitch + g.sbase;
+    int32_t* ex = tabs.expand + ((size_t)id * tabs.n_groups + grp) * kExpandCap;
 
     if (tid == 0) { mbar_init(&sh.bar[0], 1); mbar_init(&sh.bar[1], 1); sh.first_host = ne; }
     __syncthreads();
@@ -335,6 +344,18 @@ __global__ void __launch_bounds__(kTabThreads, 1) gp_build_shape_tables(Snapshot
         } else {
 #pragma unroll
             for (int j = 0; j < kTabPerThread; ++j) if (i0 + j < ne) out[i0 + j] = base + v[j];
+        }
+        // the expansion list: node i0 + j fills entries [S, S + c) of it, as far as they are below kExpandCap
+        if (base < (uint32_t)kExpandCap) {
+#pragma unroll
+            for (int j = 0; j < kTabPerThread; ++j) {
+                const uint32_t lo = base + v[j];
+                const uint32_t hi = min(base + (j + 1 < kTabPerThread ? v[j + 1] : sum), (uint32_t)kExpandCap);
+                if (lo < hi) {
+                    const int32_t node = __ldg(s.slot_node + g.sbase + i0 + j);
+                    for (uint32_t t = lo; t < hi; ++t) ex[t] = node;
+                }
+            }
         }
         carry += tile_total;
         __syncthreads();            // tile[t & 1] and part[t & 1] may be overwritten from here on
@@ -415,6 +436,13 @@ __global__ void __launch_bounds__(kDecideThreads) gp_decide_tables(Snapshot s, A
                                                                    volatile int* __restrict__ err_host, int force_scan) {
     const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     unsigned long long probes = 0, drivers = 0;
+    // placement to copy from an expansion list (see below): out[t] = list[t] for t < a, node for a <= t < a + b,
+    // list[t + skip] after that
+    bool copy = false;
+    const int32_t* list = nullptr;
+    int64_t copy_off = 0;
+    uint32_t copy_k = 0, copy_a = 0, copy_b = 0, copy_skip = 0;
+    int32_t copy_node = 0;
     if (i < n_apps) {
         const int64_t d_cpu = cols.load(0, i), d_mem = cols.load(1, i), d_gpu = cols.load(2, i);
         const int64_t e_cpu = cols.load(3, i), e_mem = cols.load(4, i), e_gpu = cols.load(5, i);
@@ -472,16 +500,16 @@ __global__ void __launch_bounds__(kDecideThreads) gp_decide_tables(Snapshot s, A
                     }
                 }
                 int32_t dslot = -1;
-                uint32_t cd = 0, c0d = 0;
+                uint32_t cd = 0, c0d = 0, spd = 0;
                 for (; j < nd; ++j) {
                     ++drivers;
                     const int32_t ls = s.drv_slot[g.dbase + j];
                     const longlong2 v = __ldg(gpair + ls);
                     const int64_t gv = (drv_gpu || cap_gpu) ? __ldg(ggpu + ls) : 0;
                     if ((d_cpu > v.x) || (d_mem > v.y) || (drv_gpu && d_gpu > gv)) continue;
-                    uint32_t my_c0 = 0, my_cd = 0;
+                    uint32_t my_c0 = 0, my_cd = 0, sp = 0;
                     if (ls < ne && k != 0) {
-                        const uint32_t sp = __ldg(tab + ls);
+                        sp = __ldg(tab + ls);
                         my_c0 = tab_at(tab, ls + 1, ne, total) - sp;
                         probes += 2;
                         if (my_c0 != 0) {        // what the node can still take once the driver sits on it
@@ -493,17 +521,27 @@ __global__ void __launch_bounds__(kDecideThreads) gp_decide_tables(Snapshot s, A
                         if (ALGO == 0 && total - (my_c0 - my_cd) < k) continue;       // the executors do not fit with this driver
                         // distribute-evenly: >= k+1 hosting nodes, the driver removes at most its own
                     }
-                    dslot = ls; cd = my_cd; c0d = my_c0;
+                    dslot = ls; cd = my_cd; c0d = my_c0; spd = sp;
                     break;
                 }
                 if (dslot >= 0) {
                     result = s.slot_node[g.sbase + dslot];
-                    if (k != 0) {
+                    if (k != 0 && k + (c0d - cd) <= (uint32_t)kExpandCap) {
+                        // ---- emission from the expansion list E: the driver's node p takes cd executors instead of
+                        // c0d, so the placement is  E[0, S[p]) ++ p x min(cd, k - S[p]) ++ E[S[p+1], ...)  when S[p] < k,
+                        // else E[0, k) (also for a driver in a spare slot).  Copied by the whole warp below.
+                        copy = true;
+                        list = tabs.expand + ((size_t)en->id * tabs.n_groups + grp) * kExpandCap;
+                        copy_off = off; copy_k = k; copy_node = result;
+                        copy_a = (dslot < ne && spd < k) ? spd : k;
+                        copy_b = min(cd, k - copy_a);
+                        copy_skip = c0d - copy_b;
+                        probes += k - copy_b;
+                    } else if (k != 0) {
                         // ---- emission: walk the prefix table from the first hosting node ---------------------------------
                         OUT* out = executor_nodes + off;
                         const int32_t* slot_node = s.slot_node + g.sbase;
                         const int32_t dpos = (dslot < ne) ? dslot : 0x7fffffff;
-                        (void)c0d;
                         int32_t pos = __ldg(tabs.first_host + (size_t)en->id * tabs.n_groups + grp);    // first node with room for the shape
                         ++probes;
                         uint32_t prev = 0, placed = 0;
@@ -561,6 +599,17 @@ __global__ void __launch_bounds__(kDecideThreads) gp_decide_tables(Snapshot s, A
                 driver_node[i] = result;
             }
         }
+    }
+    // ---- the copies, one application of the warp after the other: coalesced loads from E, coalesced stores ----------
+    const int lane = threadIdx.x & 31;
+    for (unsigned todo = __ballot_sync(kFull, copy); todo; todo &= todo - 1) {
+        const int src = __ffs(todo) - 1;
+        const int32_t* l = reinterpret_cast<const int32_t*>(__shfl_sync(kFull, reinterpret_cast<unsigned long long>(list), src));
+        OUT* out = executor_nodes + __shfl_sync(kFull, copy_off, src);
+        const uint32_t k = __shfl_sync(kFull, copy_k, src), a = __shfl_sync(kFull, copy_a, src);
+        const uint32_t ab = a + __shfl_sync(kFull, copy_b, src), skip = __shfl_sync(kFull, copy_skip, src);
+        const int32_t node = __shfl_sync(kFull, copy_node, src);
+        for (uint32_t t = lane; t < k; t += 32) out[t] = (OUT)(t < a ? __ldg(l + t) : (t < ab ? node : __ldg(l + t + skip)));
     }
     // statistics: one atomic per warp
 #pragma unroll
