@@ -12,6 +12,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -89,28 +90,22 @@ __global__ void gp_prep_apps(int32_t n_apps, AppColumns cols, const uint8_t* __r
     for (int32_t t = threadIdx.x; t < n_block * kQ; t += blockDim.x) dst[t] = stage[t];
 }
 
-// Independent mode (GP_MODE_INDEPENDENT): one warp per application; warps claim applications from a
-// global counter (claim-then-broadcast, next index prefetched) so long scans do not leave a tail.
+// Independent minimal-fragmentation (independent tightly-pack / distribute-evenly take the tables, gangpack_tables.cuh):
+// one warp per application; warps claim applications from a global counter (claim-then-broadcast, next index
+// prefetched) so long scans do not leave a tail.
 constexpr int kPackThreads = 256;
-template <int ALGO>
-#ifndef GP_PACK_MIN_BLOCKS
-#define GP_PACK_MIN_BLOCKS 4
-#endif
 #ifndef GP_MF_MIN_BLOCKS
-#define GP_MF_MIN_BLOCKS 4      // minimal-fragmentation: 64 registers (96 uncapped); measured 4.42 / 3.67 / 3.45 ms per 100 k decisions at 2 / 3 / 4 CTAs per SM
+#define GP_MF_MIN_BLOCKS 4      // 64 registers (96 uncapped); measured 4.42 / 3.67 / 3.45 ms per 100 k decisions at 2 / 3 / 4 CTAs per SM
 #endif
-__global__ void __launch_bounds__(kPackThreads, ALGO == 2 ? GP_MF_MIN_BLOCKS : GP_PACK_MIN_BLOCKS) gp_pack_independent(Snapshot s, const PrepApp* __restrict__ prep, int32_t n_apps,
+__global__ void __launch_bounds__(kPackThreads, GP_MF_MIN_BLOCKS) gp_pack_independent(Snapshot s, const PrepApp* __restrict__ prep, int32_t n_apps,
                                                                     int32_t* __restrict__ driver_node,
                                                                     int32_t* __restrict__ executor_nodes,
                                                                     int2* __restrict__ scratch,
                                                                     unsigned long long* __restrict__ stats,
                                                                     unsigned int* __restrict__ next_app) {
-    __shared__ uint16_t cap_cache[kPackThreads / 32][kCapCache];
     const int lane = threadIdx.x & 31;
-    uint16_t* wcache = cap_cache[threadIdx.x >> 5];
     WarpStats st{0, 0};
     const int snap_flags = s.meta->flags;          // per-kernel facts stay in registers
-    const GroupDesc g0 = s.groups[0];
     // claim-then-broadcast, two applications ahead: while application i is packed, the index of i+2 is in
     // flight and the record of i+1 is being pulled into L1
     unsigned int i = 0, n1 = 0;
@@ -123,14 +118,10 @@ __global__ void __launch_bounds__(kPackThreads, ALGO == 2 ? GP_MF_MIN_BLOCKS : G
         if (lane == 0 && n1 < (unsigned int)n_apps) asm volatile("prefetch.global.L1 [%0];" ::"l"(prep + n1));
         const PrepApp* pa = prep + i;
         int32_t d = -1;
-        if (!(pa->flags & kAppInvalid)) {
-            if constexpr (ALGO == 2) {       // minimal-fragmentation: multi-pass, see gangpack_minfrag.cuh
-                const bool gpu_idle = !(pa->flags & kAppUsesGpu) && !(snap_flags & kSnapGpuNegative);
-                d = ((pa->flags & kAppFast32) && gpu_idle) ? pack_app_minfrag<true>(s, pa, executor_nodes, scratch, st, lane, snap_flags)
-                                                           : pack_app_minfrag<false>(s, pa, executor_nodes, scratch, st, lane, snap_flags);
-            } else {
-                d = pack_app<ALGO, int32_t>(s, pa, executor_nodes, scratch, wcache, st, lane, snap_flags, g0);
-            }
+        if (!(pa->flags & kAppInvalid)) {        // multi-pass, see gangpack_minfrag.cuh
+            const bool gpu_idle = !(pa->flags & kAppUsesGpu) && !(snap_flags & kSnapGpuNegative);
+            d = ((pa->flags & kAppFast32) && gpu_idle) ? pack_app_minfrag<true>(s, pa, executor_nodes, scratch, st, lane, snap_flags)
+                                                       : pack_app_minfrag<false>(s, pa, executor_nodes, scratch, st, lane, snap_flags);
         }
         if (lane == 0) driver_node[i] = d;
         i = n1;
@@ -393,10 +384,8 @@ struct GraphCache {
     void reset() { if (exec) cudaGraphExecDestroy(exec); exec = nullptr; key.clear(); last_key.clear(); }
 };
 
-// dev_misc layout: [0] error bits (int), [8..24) stats (2 x u64), [32..32+4*kMaxChunks) per-chunk work counters
-static constexpr size_t kMiscCounters = 64, kMiscBytes = 64 + 4 * 16;   // [0] err, [8..40) 4 x u64 statistics, [64..) counters
-static constexpr int32_t kChunkApps = 50000;
-static constexpr int32_t kZeroCopyOutApps = 8192;  // batches up to this size write results straight into mapped host memory   // apps per pipelined chunk of gp_pack_batch (~1.5 MB H2D, ~70 us of kernel)
+static constexpr int32_t kChunkApps = 50000;       // apps per pipelined chunk of gp_pack_batch (~1.5 MB H2D, ~70 us of kernel)
+static constexpr int32_t kZeroCopyOutApps = 8192;  // batches up to this size write results straight into mapped host memory
 
 struct gp_ctx {
     int device = 0;
@@ -404,6 +393,19 @@ struct gp_ctx {
     cudaStream_t stream = nullptr;
     static constexpr int kLanes = 3;       // H2D / kernels / D2H of consecutive chunks overlap across lanes
     static constexpr int kMaxChunks = 16;
+    // what the kernels of one pack call report; pack_begin zeroes all of it with one memset
+    struct DevStatus {
+        int err;                              // kErr* bits
+        unsigned long long stats[4];          // nodes scanned, drivers tried, scan-path applications, scan-path nodes
+        unsigned int fifo_cursor;             // gp_pack_fifo_cta: next application in queue order
+        unsigned int next_app[kMaxChunks];    // per pipelined chunk: next application claimed by the persistent pack kernels
+    };
+    // pinned host mirror: gp_last_stats copies the err / stats prefix of DevStatus into `dev`; the kernels also set
+    // `err_word` through the mapping, so a pack call reads its validation errors after the stream sync without a copy
+    struct HostStatus {
+        DevStatus dev;
+        volatile int err_word;
+    };
     cudaStream_t lane[kLanes] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev[kMaxChunks][3] = {};    // per chunk: prep start, pack start, pack end
     cudaEvent_t ev_ready = nullptr, ev_done[kLanes] = {nullptr, nullptr, nullptr};
@@ -420,10 +422,11 @@ struct gp_ctx {
     DevBuf snap_aux;                              // slot layout scratch (build_snapshot_device)
 
     // batch staging
-    DevBuf a_dcpu, a_dmem, a_dgpu, a_ecpu, a_emem, a_egpu, a_count, a_group, a_skip, a_off;
-    DevBuf prep, r_driver, r_exec, scratch, dev_misc, gmin, sortbuf, usagebuf, reschedbuf;
-    std::vector<int32_t> iota;   // dev_misc: [0] err int, [2..3] stats u64 x2 (8B aligned at +8)
-    void* pinned_misc = nullptr;                         // 32 B pinned mirror of dev_misc
+    DevBuf a_quant, a_count, a_group, a_skip, a_off;   // a_quant: the six quantity columns, one pitched block
+    DevBuf prep, r_driver, r_exec, scratch, gmin, sortbuf, usagebuf, reschedbuf;
+    DevBuf status;                                // one DevStatus; never reallocated, so its address can key a graph
+    HostStatus* status_host = nullptr;
+    DevStatus* dev_status() const { return status.as<DevStatus>(); }
     std::vector<int64_t> host_off;
     std::vector<int32_t> v_owner;                 // gp_set_snapshot validation scratch (no per-call allocation)
     std::vector<uint8_t> v_seen_e, v_seen_d;
@@ -435,7 +438,7 @@ struct gp_ctx {
     bool async_snapshot = false;                  // gp_config.flags & GP_CFG_ASYNC_SNAPSHOT
     int chunk_apps = kChunkApps;                  // GANGPACK_CHUNK_APPS
     int trace = 0;                                // GANGPACK_TRACE=1: host-side phase timing on stderr
-    int pack_ctas_per_sm[3] = {0, 0, 0};            // occupancy of gp_pack_independent<ALGO> on this device
+    int pack_ctas_per_sm = 0;                       // occupancy of gp_pack_independent on this device
     int tab_ctas_per_sm[2][2] = {{0, 0}, {0, 0}};   // occupancy of gp_pack_tables<ALGO, OUT>
     bool tab_attr_set[2] = {false, false};
     // per pipeline lane: shape hash + header, capacity tables, group totals, expansion lists, per-application shape slot
@@ -540,6 +543,24 @@ static gp_status fail(gp_ctx* ctx, gp_status st, const std::string& msg) {
     return st;
 }
 
+// Staging of the auxiliary entry points: stage() lays out every part(pointer, count) in one DevBuf, each sub-buffer
+// 256-byte aligned, reserves the DevBuf once and points every pointer at its sub-buffer.  The same counts give the
+// same addresses from one call to the next.
+template <class T> struct Part { T** p; size_t n; };
+template <class T> static Part<T> part(T*& p, size_t n) { return Part<T>{&p, n}; }
+static size_t part_bytes(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
+template <class... T> static cudaError_t stage(DevBuf& buf, Part<T>... parts) {
+    const cudaError_t e = buf.reserve((part_bytes(sizeof(T) * parts.n) + ... + 0));
+    if (e != cudaSuccess) return e;
+    char* at = buf.as<char>();
+    ((*parts.p = reinterpret_cast<T*>(at), at += part_bytes(sizeof(T) * parts.n)), ...);
+    return cudaSuccess;
+}
+// host -> device copy into a staged part; a NULL source (an optional column left out) copies nothing
+static cudaError_t upload(void* dst, const void* src, size_t bytes, cudaStream_t st) {
+    return src ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess;
+}
+
 static Snapshot make_snapshot(const gp_ctx* c) {
     Snapshot s;
     s.pair = c->pair.as<longlong2>();
@@ -596,15 +617,17 @@ gp_status gp_create(gp_ctx** out, const gp_config* cfg) {
     if (const char* z = std::getenv("GANGPACK_GRAPHS")) c->use_graphs = std::atoi(z);
     if (const char* z = std::getenv("GANGPACK_CHUNK_APPS")) c->chunk_apps = std::max(1024, std::atoi(z));
     if (const char* z = std::getenv("GANGPACK_TRACE")) c->trace = std::atoi(z);
+    void* status_host = nullptr;
     if ((e = cudaSetDevice(dev)) != cudaSuccess ||
         (e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)) != cudaSuccess ||
         (e = create_aux(c)) != cudaSuccess ||
-        (e = cudaHostAlloc(&c->pinned_misc, 64, cudaHostAllocDefault)) != cudaSuccess ||
-        (e = c->dev_misc.reserve(kMiscBytes)) != cudaSuccess || (e = c->snap_flags.reserve(sizeof(SnapMeta))) != cudaSuccess) {
+        (e = cudaHostAlloc(&status_host, sizeof(gp_ctx::HostStatus), cudaHostAllocDefault)) != cudaSuccess ||
+        (e = c->status.reserve(sizeof(gp_ctx::DevStatus))) != cudaSuccess || (e = c->snap_flags.reserve(sizeof(SnapMeta))) != cudaSuccess) {
         g_create_error = std::string("gp_create: ") + cudaGetErrorString(e);
         delete c;
         return GP_ERR_CUDA;
     }
+    c->status_host = static_cast<gp_ctx::HostStatus*>(status_host);
     *out = c;
     return GP_OK;
 }
@@ -615,14 +638,13 @@ void gp_destroy(gp_ctx* c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     DevBuf* bufs[] = {&c->node_cpu, &c->node_mem, &c->node_gpu, &c->exec_off, &c->drv_off, &c->exec_order, &c->drv_order,
                       &c->pair, &c->pair32, &c->sgpu, &c->slot_node, &c->node_slot, &c->drv_slot, &c->groups, &c->snap_flags, &c->snap_aux,
-                      &c->a_dcpu, &c->a_dmem, &c->a_dgpu, &c->a_ecpu, &c->a_emem, &c->a_egpu, &c->a_count, &c->a_group,
-                      &c->a_skip, &c->a_off, &c->prep, &c->r_driver, &c->r_exec, &c->scratch, &c->dev_misc, &c->gmin, &c->sortbuf, &c->usagebuf, &c->reschedbuf,
-                      &c->off_dev, &c->fifo_list, &c->sched, &c->zonebuf};
+                      &c->a_quant, &c->a_count, &c->a_group, &c->a_skip, &c->a_off, &c->prep, &c->r_driver, &c->r_exec, &c->scratch,
+                      &c->gmin, &c->sortbuf, &c->usagebuf, &c->reschedbuf, &c->status, &c->off_dev, &c->fifo_list, &c->sched, &c->zonebuf};
     for (DevBuf* b : bufs) b->release();
     for (auto& t : c->tabs) { t.hdr.release(); t.table.release(); t.total.release(); t.expand.release(); t.app_slot.release(); }
     for (auto& g : c->g_chunk) g.reset();
     c->g_snapshot.reset();
-    if (c->pinned_misc) cudaFreeHost(c->pinned_misc);
+    if (c->status_host) cudaFreeHost(c->status_host);
     if (c->one_block) cudaFreeHost(c->one_block);
     for (auto& row : c->ev) for (cudaEvent_t e : row) if (e) cudaEventDestroy(e);
     if (c->ev_ready) cudaEventDestroy(c->ev_ready);
@@ -890,20 +912,20 @@ template <int ALGO>
 static void launch_pack(gp_ctx* c, gp_mode mode, const Snapshot& s, const PrepApp* prep, const int32_t* app_group, int32_t n_apps,
                         int32_t* driver_node, int32_t* executor_nodes, int2* scratch, unsigned long long* stats,
                         unsigned int* next_app, cudaStream_t st) {
-    if (mode == GP_MODE_INDEPENDENT) {
+    if constexpr (ALGO == 2) {     // minimal-fragmentation: GP_MODE_INDEPENDENT only (check_args)
         // persistent grid: as many CTAs as fit on the device (or fewer for small batches)
-        int& per_sm = c->pack_ctas_per_sm[ALGO];
+        int& per_sm = c->pack_ctas_per_sm;
         if (per_sm == 0) {
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gp_pack_independent<ALGO>, kPackThreads, 0);
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gp_pack_independent, kPackThreads, 0);
             if (per_sm < 1) per_sm = 1;
         }
         int64_t blocks = ((int64_t)n_apps * 32 + kPackThreads - 1) / kPackThreads;
         int64_t max_blocks = (int64_t)c->sm_count * per_sm;
         if (blocks > max_blocks) blocks = max_blocks;
         if (blocks < 1) blocks = 1;
-        gp_pack_independent<ALGO><<<(int)blocks, kPackThreads, 0, st>>>(s, prep, n_apps, driver_node, executor_nodes, scratch,
-                                                                       stats, next_app);
-    } else if constexpr (ALGO != 2) {     // (check_args rejects the FIFO modes for minimal-fragmentation)
+        gp_pack_independent<<<(int)blocks, kPackThreads, 0, st>>>(s, prep, n_apps, driver_node, executor_nodes, scratch,
+                                                                 stats, next_app);
+    } else {                       // tightly-pack / distribute-evenly come here in the FIFO modes only (launch_tables)
         // FIFO: one persistent 1024-thread CTA per instance group, its slots staged in shared memory
         bool& attr_set = c->fifo_attr_set[ALGO];     // per device: function attributes live in the device's context
         if (!attr_set) {
@@ -911,16 +933,12 @@ static void launch_pack(gp_ctx* c, gp_mode mode, const Snapshot& s, const PrepAp
             cudaFuncSetAttribute(gp_pack_fifo_cta<ALGO, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFifoSmemBytes);
             attr_set = true;
         }
-        // small groups: fewer threads per CTA (the per-application fixed cost scales with the CTA size)
-        const int avg_ne = c->n_groups > 0 ? c->n_exec / c->n_groups : 0;
-        const int kFifoThreadsRt = kFifoThreads;
-        (void)avg_ne;
         int32_t* app_list = c->fifo_list.as<int32_t>();
-        unsigned int* cursor = reinterpret_cast<unsigned int*>(c->dev_misc.as<char>() + 56);     // zeroed by pack_begin
+        unsigned int* cursor = &c->dev_status()->fifo_cursor;
         if (mode == GP_MODE_FIFO_REFERENCE)
-            gp_pack_fifo_cta<ALGO, 1><<<s.n_groups, kFifoThreadsRt, kFifoSmemBytes, st>>>(s, prep, app_group, n_apps, driver_node, executor_nodes, scratch, stats, s.gmins, app_list, cursor);
+            gp_pack_fifo_cta<ALGO, 1><<<s.n_groups, kFifoThreads, kFifoSmemBytes, st>>>(s, prep, app_group, n_apps, driver_node, executor_nodes, scratch, stats, s.gmins, app_list, cursor);
         else
-            gp_pack_fifo_cta<ALGO, 2><<<s.n_groups, kFifoThreadsRt, kFifoSmemBytes, st>>>(s, prep, app_group, n_apps, driver_node, executor_nodes, scratch, stats, s.gmins, app_list, cursor);
+            gp_pack_fifo_cta<ALGO, 2><<<s.n_groups, kFifoThreads, kFifoSmemBytes, st>>>(s, prep, app_group, n_apps, driver_node, executor_nodes, scratch, stats, s.gmins, app_list, cursor);
         // the FIFO kernels subtract usage from `pair` in place: refresh the compact 32-bit view so that a later
         // independent pack on this context (the driver's own pack after fitEarlierDrivers, resource.go:255 then :321)
         // sees the charged availability
@@ -971,10 +989,11 @@ static gp_status pack_device_range(gp_ctx* c, const DevApps& da, int32_t lo, int
                                    const DevResults& dr, int2* scratch, cudaStream_t st, int chunk) {
     const int32_t q = hi - lo;
     if (q <= 0) return GP_OK;
-    int* d_err = c->dev_misc.as<int>();
-    unsigned long long* d_stats = reinterpret_cast<unsigned long long*>(c->dev_misc.as<char>() + 8);
-    unsigned int* next_app = reinterpret_cast<unsigned int*>(c->dev_misc.as<char>() + kMiscCounters) + chunk;
-    volatile int* err_host = reinterpret_cast<volatile int*>(static_cast<char*>(c->pinned_misc) + 48);
+    gp_ctx::DevStatus* ds = c->dev_status();
+    int* d_err = &ds->err;
+    unsigned long long* d_stats = ds->stats;
+    unsigned int* next_app = ds->next_app + chunk;
+    volatile int* err_host = &c->status_host->err_word;
     Snapshot s = make_snapshot(c);
     AppColumns cols = cols_at(da.cols, lo);
 
@@ -1085,8 +1104,8 @@ static bool fused_path(gp_algo algo, gp_mode mode) { return mode == GP_MODE_INDE
 
 // common prologue: buffers, counters
 static gp_status pack_begin(gp_ctx* c, int32_t q, gp_algo algo, gp_mode mode, int64_t exec_cap, bool derive_off, int2** scratch, cudaStream_t st) {
-    GP_CUDA(c, cudaMemsetAsync(c->dev_misc.p, 0, kMiscBytes, st));
-    *reinterpret_cast<volatile int*>(static_cast<char*>(c->pinned_misc) + 48) = 0;   // host-visible error word
+    GP_CUDA(c, cudaMemsetAsync(c->status.p, 0, sizeof(gp_ctx::DevStatus), st));
+    c->status_host->err_word = 0;
     c->last = gp_stats{};
     c->ev_chunks = 0;
     *scratch = nullptr;
@@ -1140,6 +1159,9 @@ static gp_status decode_device_error(gp_ctx* c, int err) {
     return fail(c, GP_ERR_CAPACITY, "pack: exec_out_off inconsistent with exe_count or executor_nodes_cap too small");
 }
 
+// the validation errors of the pack call just synchronised, from the host-visible error word
+static gp_status pack_error(gp_ctx* c) { return decode_device_error(c, c->status_host->err_word); }
+
 static gp_apps_wire widen(const gp_apps* a) {
     gp_apps_wire w{};
     w.n_apps = a->n_apps; w.quantity_bits = 64; w.mem_shift = 0;
@@ -1177,17 +1199,16 @@ gp_status gp_pack_batch_device(gp_ctx* c, const gp_apps* da, gp_algo algo, gp_mo
 gp_status gp_last_stats(gp_ctx* c, gp_stats* out) {
     if (!c || !out) return GP_ERR_INVALID;
     GP_CUDA(c, cudaSetDevice(c->device));
-    GP_CUDA(c, cudaMemcpyAsync(c->pinned_misc, c->dev_misc.p, 40, cudaMemcpyDeviceToHost, c->stream));
+    gp_ctx::DevStatus& h = c->status_host->dev;
+    GP_CUDA(c, cudaMemcpyAsync(&h, c->status.p, offsetof(gp_ctx::DevStatus, stats) + sizeof(h.stats), cudaMemcpyDeviceToHost, c->stream));
     GP_CUDA(c, cudaStreamSynchronize(c->stream));
-    const unsigned long long* s = reinterpret_cast<const unsigned long long*>((const char*)c->pinned_misc + 8);
-    c->last.nodes_scanned = (int64_t)s[0];
-    c->last.drivers_tried = (int64_t)s[1];
-    c->last.scan_path_apps = (int64_t)s[2];
-    c->last.scan_path_nodes = (int64_t)s[3];
+    c->last.nodes_scanned = (int64_t)h.stats[0];
+    c->last.drivers_tried = (int64_t)h.stats[1];
+    c->last.scan_path_apps = (int64_t)h.stats[2];
+    c->last.scan_path_nodes = (int64_t)h.stats[3];
     fill_kernel_times(c);
     *out = c->last;
-    int err = *reinterpret_cast<const int*>(c->pinned_misc);
-    return decode_device_error(c, err);
+    return decode_device_error(c, h.err);
 }
 
 static gp_status pack_batch_impl(gp_ctx* c, const gp_apps_wire* a, gp_algo algo, gp_mode mode, gp_results_wire* out);
@@ -1236,7 +1257,7 @@ static gp_status pack_batch_impl(gp_ctx* c, const gp_apps_wire* a, gp_algo algo,
     // the quantity columns are staged in ONE pitched device block (rows: drv cpu, drv mem, exe cpu, exe mem, drv gpu,
     // exe gpu) so that equally spaced host columns can be moved by a single 2-D DMA per chunk
     const size_t dpitch = (bq + 255) & ~(size_t)255;
-    GP_CUDA(c, c->a_dcpu.reserve(dpitch * 6));
+    GP_CUDA(c, c->a_quant.reserve(dpitch * 6));
     GP_CUDA(c, c->a_count.reserve(b32));
     if (off) GP_CUDA(c, c->a_off.reserve(sizeof(int64_t) * (size_t)(q + 1)));
     GP_CUDA(c, c->r_driver.reserve(b32));
@@ -1250,7 +1271,7 @@ static gp_status pack_batch_impl(gp_ctx* c, const gp_apps_wire* a, gp_algo algo,
     void* mo_driver = small ? const_cast<void*>(mapped_ptr(c, out->driver_node, b32)) : nullptr;
     void* mo_exec = (small && out->executor_nodes) ? const_cast<void*>(mapped_ptr(c, out->executor_nodes, os * (size_t)out->executor_nodes_cap)) : nullptr;
     const bool out_mapped = small && mo_driver && (out->executor_nodes_cap == 0 || !out->executor_nodes || mo_exec);
-    char* blk = c->a_dcpu.as<char>();
+    char* blk = c->a_quant.as<char>();
     DevApps dv{};
     const void* hq[6] = {a->drv_cpu, a->drv_mem, a->exe_cpu, a->exe_mem, a->drv_gpu, a->exe_gpu};    // staging row order
     dv.cols.q[0] = blk + 0 * dpitch; dv.cols.q[1] = blk + 1 * dpitch; dv.cols.q[3] = blk + 2 * dpitch; dv.cols.q[4] = blk + 3 * dpitch;
@@ -1391,7 +1412,7 @@ static gp_status pack_batch_impl(gp_ctx* c, const gp_apps_wire* a, gp_algo algo,
     }
     // validation errors arrive through the mapped error word; scan statistics stay on the device until
     // gp_last_stats asks for them
-    return decode_device_error(c, *reinterpret_cast<volatile int*>(static_cast<char*>(c->pinned_misc) + 48));
+    return pack_error(c);
 }
 
 gp_status gp_pack_one(gp_ctx* c, gp_algo algo, int64_t drv_cpu, int64_t drv_mem, int64_t drv_gpu, int64_t exe_cpu,
@@ -1461,24 +1482,70 @@ gp_status gp_set_schedulable(gp_ctx* c, const int64_t* cpu, const int64_t* mem, 
     return GP_OK;
 }
 
+// the checks the two single-AZ entry points run first
+static gp_status check_zone_call(gp_ctx* c, const gp_apps* a, const gp_zone_results* out, const char* who) {
+    if (!c->have_snapshot) return fail(c, GP_ERR_NO_SNAPSHOT, std::string(who) + ": gp_set_snapshot first");
+    if (!c->have_sched) return fail(c, GP_ERR_INVALID, std::string(who) + ": gp_set_schedulable first (the efficiencies need SchedulableResources)");
+    if (!a || !out || a->n_apps < 0) return fail(c, GP_ERR_INVALID, std::string(who) + ": NULL apps/results");
+    return GP_OK;
+}
+
+static bool has_requests(const gp_apps* a) {
+    return a->drv_cpu_milli && a->drv_mem_bytes && a->exe_cpu_milli && a->exe_mem_bytes && a->exe_count;
+}
+
+// c->host_off = exclusive prefix sum of the executor counts (negative counts as 0); returns the largest count, at least 1
+static int64_t count_offsets(gp_ctx* c, const gp_apps* a) {
+    std::vector<int64_t>& off = c->host_off;
+    off.resize((size_t)a->n_apps + 1);
+    int64_t acc = 0, widest = 1;
+    for (int32_t i = 0; i < a->n_apps; ++i) {
+        const int64_t k = a->exe_count[i] > 0 ? a->exe_count[i] : 0;
+        off[(size_t)i] = acc; acc += k;
+        if (k > widest) widest = k;
+    }
+    off[(size_t)a->n_apps] = acc;
+    return widest;
+}
+
+// the six int64 request columns into req[6][q] (a gpu column not given stays NULL in `cols`), the executor counts and
+// the [q + 1] ExecutorNodes offsets `off`
+static gp_status upload_apps(gp_ctx* c, const gp_apps* a, const int64_t* off, size_t q, cudaStream_t st, int64_t* req, int32_t* cnt,
+                             int64_t* d_off, SixCols& cols) {
+    const int64_t* hc[6] = {a->drv_cpu_milli, a->drv_mem_bytes, a->drv_gpu, a->exe_cpu_milli, a->exe_mem_bytes, a->exe_gpu};
+    for (int k = 0; k < 6; ++k) {
+        GP_CUDA(c, upload(req + q * (size_t)k, hc[k], 8 * q, st));
+        cols.p[k] = hc[k] ? req + q * (size_t)k : nullptr;
+    }
+    GP_CUDA(c, upload(cnt, a->exe_count, 4 * q, st));
+    GP_CUDA(c, upload(d_off, off, 8 * (q + 1), st));
+    return GP_OK;
+}
+
+// results of a single-AZ call to the host; after the stream sync, the validation errors of its pack
+static gp_status zone_results_back(gp_ctx* c, gp_zone_results* out, const int32_t* zone, const int32_t* driver, const int32_t* exec,
+                                   const double* avg, size_t q, size_t total, cudaStream_t st) {
+    GP_CUDA(c, cudaMemcpyAsync(out->zone, zone, 4 * q, cudaMemcpyDeviceToHost, st));
+    GP_CUDA(c, cudaMemcpyAsync(out->driver_node, driver, 4 * q, cudaMemcpyDeviceToHost, st));
+    if (total) GP_CUDA(c, cudaMemcpyAsync(out->executor_nodes, exec, 4 * total, cudaMemcpyDeviceToHost, st));
+    if (out->avg_efficiency) GP_CUDA(c, cudaMemcpyAsync(out->avg_efficiency, avg, 32 * q, cudaMemcpyDeviceToHost, st));
+    GP_CUDA(c, cudaStreamSynchronize(st));
+    return pack_error(c);
+}
+
 gp_status gp_pack_batch_zones(gp_ctx* c, const gp_apps* a, gp_algo algo, gp_zone_results* out) {
     if (!c) return GP_ERR_INVALID;
-    if (!c->have_snapshot) return fail(c, GP_ERR_NO_SNAPSHOT, "gp_pack_batch_zones: gp_set_snapshot first");
-    if (!c->have_sched) return fail(c, GP_ERR_INVALID, "gp_pack_batch_zones: gp_set_schedulable first (the efficiencies need SchedulableResources)");
-    if (!a || !out || a->n_apps < 0) return fail(c, GP_ERR_INVALID, "gp_pack_batch_zones: NULL apps/results");
+    gp_status s = check_zone_call(c, a, out, "gp_pack_batch_zones");
+    if (s != GP_OK) return s;
     if (algo != GP_TIGHTLY_PACK && algo != GP_MINIMAL_FRAGMENTATION)
         return fail(c, GP_ERR_INVALID, "gp_pack_batch_zones: the single-AZ packers are tightly-pack and minimal-fragmentation (single_az_pack_tightly.go, single_az_minimal_fragmentation.go)");
     const int32_t Q = a->n_apps, Z = c->n_groups;
     if (Q == 0) return GP_OK;
-    if (!a->drv_cpu_milli || !a->drv_mem_bytes || !a->exe_cpu_milli || !a->exe_mem_bytes || !a->exe_count || !out->zone || !out->driver_node)
-        return fail(c, GP_ERR_INVALID, "gp_pack_batch_zones: missing app/result arrays");
+    if (!has_requests(a) || !out->zone || !out->driver_node) return fail(c, GP_ERR_INVALID, "gp_pack_batch_zones: missing app/result arrays");
     if ((int64_t)Q * Z > 0x7fffffffLL) return fail(c, GP_ERR_INVALID, "gp_pack_batch_zones: n_apps x zones too large");
     const int64_t* off = a->exec_out_off;
     if (!off) {
-        c->host_off.resize((size_t)Q + 1);
-        int64_t acc = 0;
-        for (int32_t i = 0; i < Q; ++i) { c->host_off[(size_t)i] = acc; acc += a->exe_count[i] > 0 ? a->exe_count[i] : 0; }
-        c->host_off[(size_t)Q] = acc;
+        count_offsets(c, a);
         off = c->host_off.data();
     }
     const int64_t total = off[Q];
@@ -1487,38 +1554,30 @@ gp_status gp_pack_batch_zones(gp_ctx* c, const gp_apps* a, gp_algo algo, gp_zone
     GP_CUDA(c, cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
     const size_t q = (size_t)Q, R = q * (size_t)Z, T = (size_t)total;
-    size_t o = 0;
-    auto take = [&](size_t bytes) { size_t r = o; o += (bytes + 255) & ~(size_t)255; return r; };
-    const size_t o_in = take(48 * q), o_cnt = take(4 * q), o_off = take(8 * (q + 1)), o_rows = take(48 * R), o_rcnt = take(4 * R), o_rgrp = take(4 * R),
-                 o_roff = take(8 * (R + 1)), o_rdrv = take(4 * R), o_rexe = take(4 * ((size_t)Z * T + 1)), o_zone = take(4 * q), o_drv = take(4 * q),
-                 o_exe = take(4 * (T + 1)), o_avg = take(32 * q);
-    GP_CUDA(c, c->zonebuf.reserve(o));
-    char* b = c->zonebuf.as<char>();
-    const int64_t* hc[6] = {a->drv_cpu_milli, a->drv_mem_bytes, a->drv_gpu, a->exe_cpu_milli, a->exe_mem_bytes, a->exe_gpu};
+    int64_t *in, *d_off, *rows, *roff;
+    int32_t *cnt, *rcnt, *rgrp, *rdrv, *rexe, *zone, *drv, *exe;
+    double* avg;
+    GP_CUDA(c, stage(c->zonebuf, part(in, 6 * q), part(cnt, q), part(d_off, q + 1), part(rows, 6 * R), part(rcnt, R), part(rgrp, R),
+                     part(roff, R + 1), part(rdrv, R), part(rexe, (size_t)Z * T + 1), part(zone, q), part(drv, q), part(exe, T + 1),
+                     part(avg, 4 * q)));
     SixCols six{};
-    for (int k = 0; k < 6; ++k) {
-        if (!hc[k]) continue;
-        GP_CUDA(c, cudaMemcpyAsync(b + o_in + 8 * q * (size_t)k, hc[k], 8 * q, cudaMemcpyHostToDevice, st));
-        six.p[k] = reinterpret_cast<const int64_t*>(b + o_in + 8 * q * (size_t)k);
-    }
-    GP_CUDA(c, cudaMemcpyAsync(b + o_cnt, a->exe_count, 4 * q, cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(b + o_off, off, 8 * (q + 1), cudaMemcpyHostToDevice, st));
+    s = upload_apps(c, a, off, q, st, in, cnt, d_off, six);
+    if (s != GP_OK) return s;
     const int TH = 256;
     // the efficiencies read the availability in node-table order: refresh that copy from the slots (a FIFO batch may
     // have charged them since gp_set_snapshot)
     if (c->n_slots > 0)
         gp_scatter_slots<<<(c->n_slots + TH - 1) / TH, TH, 0, st>>>(c->n_slots, c->pair.as<longlong2>(), c->sgpu.as<int64_t>(), c->slot_node.as<int32_t>(),
                                                                    c->node_cpu.as<int64_t>(), c->node_mem.as<int64_t>(), c->node_gpu.as<int64_t>());
-    gp_zone_expand<<<(unsigned)((R + 1 + TH - 1) / TH), TH, 0, st>>>(Q, Z, six, (const int32_t*)(b + o_cnt), (const int64_t*)(b + o_off),
-                                                                      (int64_t*)(b + o_rows), (int32_t*)(b + o_rcnt), (int32_t*)(b + o_rgrp), (int64_t*)(b + o_roff));
+    gp_zone_expand<<<(unsigned)((R + 1 + TH - 1) / TH), TH, 0, st>>>(Q, Z, six, cnt, d_off, rows, rcnt, rgrp, roff);
     int2* scratch = nullptr;
-    gp_status s = pack_begin(c, (int32_t)R, algo, GP_MODE_INDEPENDENT, (int64_t)Z * total, false, &scratch, st);
+    s = pack_begin(c, (int32_t)R, algo, GP_MODE_INDEPENDENT, (int64_t)Z * total, false, &scratch, st);
     if (s != GP_OK) return s;
     DevApps dv{};
-    for (int k = 0; k < 6; ++k) dv.cols.q[k] = b + o_rows + 8 * R * (size_t)k;
-    dv.cols.count = (const int32_t*)(b + o_rcnt); dv.cols.group = (const int32_t*)(b + o_rgrp); dv.cols.off = (const int64_t*)(b + o_roff);
+    for (int k = 0; k < 6; ++k) dv.cols.q[k] = rows + R * (size_t)k;
+    dv.cols.count = rcnt; dv.cols.group = rgrp; dv.cols.off = roff;
     dv.cols.bits = 64; dv.cols.mem_shift = 0; dv.skip = nullptr; dv.n = (int32_t)R;
-    DevResults dr{(int32_t*)(b + o_rdrv), b + o_rexe, (int64_t)Z * total, 32};
+    DevResults dr{rdrv, rexe, (int64_t)Z * total, 32};
     s = pack_device_range(c, dv, 0, (int32_t)R, 0, algo, GP_MODE_INDEPENDENT, dr, scratch, st, 0);
     if (s != GP_OK) return s;
     c->ev_chunks = 1;
@@ -1527,32 +1586,23 @@ gp_status gp_pack_batch_zones(gp_ctx* c, const gp_apps* a, gp_algo algo, gp_zone
     zi.avail[0] = c->node_cpu.as<long long>(); zi.avail[1] = c->node_mem.as<long long>(); zi.avail[2] = c->node_gpu.as<long long>();
     zi.sched[0] = c->sched.as<long long>(); zi.sched[1] = c->sched.as<long long>() + N; zi.sched[2] = c->sched.as<long long>() + 2 * N;
     for (int k = 0; k < 3; ++k) { zi.drv[k] = six.p[k]; zi.exe[k] = six.p[3 + k]; }
-    zi.count = (const int32_t*)(b + o_cnt); zi.out_off = (const int64_t*)(b + o_off);
-    zi.row_driver = (const int32_t*)(b + o_rdrv); zi.row_exec = (const int32_t*)(b + o_rexe);
+    zi.count = cnt; zi.out_off = d_off;
+    zi.row_driver = rdrv; zi.row_exec = rexe;
     zi.n_apps = Q; zi.n_zones = Z; zi.executors_reserved = algo == GP_TIGHTLY_PACK ? 1 : 0;
-    gp_zone_choose<<<(unsigned)((q * 32 + TH - 1) / TH), TH, 0, st>>>(zi, (int32_t*)(b + o_zone), (int32_t*)(b + o_drv), (int32_t*)(b + o_exe),
-                                                                       out->avg_efficiency ? (double*)(b + o_avg) : nullptr);
+    gp_zone_choose<<<(unsigned)((q * 32 + TH - 1) / TH), TH, 0, st>>>(zi, zone, drv, exe, out->avg_efficiency ? avg : nullptr);
     GP_CUDA(c, cudaGetLastError());
     c->last.kernel_launches += 2;
-    GP_CUDA(c, cudaMemcpyAsync(out->zone, b + o_zone, 4 * q, cudaMemcpyDeviceToHost, st));
-    GP_CUDA(c, cudaMemcpyAsync(out->driver_node, b + o_drv, 4 * q, cudaMemcpyDeviceToHost, st));
-    if (T) GP_CUDA(c, cudaMemcpyAsync(out->executor_nodes, b + o_exe, 4 * T, cudaMemcpyDeviceToHost, st));
-    if (out->avg_efficiency) GP_CUDA(c, cudaMemcpyAsync(out->avg_efficiency, b + o_avg, 32 * q, cudaMemcpyDeviceToHost, st));
-    GP_CUDA(c, cudaStreamSynchronize(st));
-    return decode_device_error(c, *reinterpret_cast<volatile int*>(static_cast<char*>(c->pinned_misc) + 48));
+    return zone_results_back(c, out, zone, drv, exe, avg, q, T, st);
 }
 
 // ---- reservation table + device-resident snapshot upkeep (gangpack_zones.cuh) -------------------------------------------
-static gp_status refresh_views(gp_ctx* c, bool raised, cudaStream_t st) {
+// the snapshot-wide facts and the compact view after availabilities changed in place
+static gp_status refresh_views(gp_ctx* c, cudaStream_t st) {
     const int T = 256;
     if (c->n_slots <= 0) return GP_OK;
     SnapMeta* meta = c->snap_flags.as<SnapMeta>();
-    if (raised)
-        gp_refresh_meta<<<(c->n_slots + T - 1) / T, T, 0, st>>>(c->n_slots, c->pair.as<longlong2>(), c->sgpu.as<long long>(), c->slot_node.as<int32_t>(),
-                                                               &meta->flags, meta->max_avail);
-    else   // availabilities only went down: a negative gpu value may have appeared
-        gp_refresh_meta<<<(c->n_slots + T - 1) / T, T, 0, st>>>(c->n_slots, c->pair.as<longlong2>(), c->sgpu.as<long long>(), c->slot_node.as<int32_t>(),
-                                                               &meta->flags, meta->max_avail);
+    gp_refresh_meta<<<(c->n_slots + T - 1) / T, T, 0, st>>>(c->n_slots, c->pair.as<longlong2>(), c->sgpu.as<long long>(), c->slot_node.as<int32_t>(),
+                                                           &meta->flags, meta->max_avail);
     gp_fill_pair32<<<(c->n_slots + T) / T, T, 0, st>>>(c->n_slots, c->pair.as<longlong2>(), meta, c->pair32.as<uint2>());
     GP_CUDA(c, cudaGetLastError());
     return GP_OK;
@@ -1561,9 +1611,8 @@ static gp_status refresh_views(gp_ctx* c, bool raised, cudaStream_t st) {
 // the FIFO loop with a single-AZ packer in one launch (gangpack_zonefifo.cuh)
 gp_status gp_pack_fifo_zones(gp_ctx* c, const gp_apps* a, gp_algo algo, gp_mode mode, gp_zone_results* out) {
     if (!c) return GP_ERR_INVALID;
-    if (!c->have_snapshot) return fail(c, GP_ERR_NO_SNAPSHOT, "gp_pack_fifo_zones: gp_set_snapshot first");
-    if (!c->have_sched) return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: gp_set_schedulable first (the efficiencies need SchedulableResources)");
-    if (!a || !out || a->n_apps < 0) return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: NULL apps/results");
+    gp_status s = check_zone_call(c, a, out, "gp_pack_fifo_zones");
+    if (s != GP_OK) return s;
     if (algo != GP_TIGHTLY_PACK && algo != GP_MINIMAL_FRAGMENTATION)
         return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: the single-AZ packers are tightly-pack and minimal-fragmentation");
     if (mode != GP_MODE_FIFO_REFERENCE && mode != GP_MODE_FIFO_EXACT)
@@ -1571,81 +1620,62 @@ gp_status gp_pack_fifo_zones(gp_ctx* c, const gp_apps* a, gp_algo algo, gp_mode 
     const int32_t Q = a->n_apps, Z = c->n_groups;
     if (Z > kZoneFifoMaxZones) return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: more than 64 zones");
     if (Q == 0) return GP_OK;
-    if (!a->drv_cpu_milli || !a->drv_mem_bytes || !a->exe_cpu_milli || !a->exe_mem_bytes || !a->exe_count || !out->zone || !out->driver_node)
-        return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: missing app/result arrays");
-    std::vector<int64_t>& hoff = c->host_off;
-    hoff.resize((size_t)Q + 1);
-    int64_t acc = 0, pitch = 1;
-    for (int32_t i = 0; i < Q; ++i) {
-        const int64_t k = a->exe_count[i] > 0 ? a->exe_count[i] : 0;
-        hoff[(size_t)i] = acc; acc += k;
-        if (k > pitch) pitch = k;
-    }
-    hoff[(size_t)Q] = acc;
+    if (!has_requests(a) || !out->zone || !out->driver_node) return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: missing app/result arrays");
+    int64_t pitch = count_offsets(c, a);
+    const std::vector<int64_t>& hoff = c->host_off;
     if (a->exec_out_off)
         for (int32_t i = 0; i <= Q; ++i)
             if (a->exec_out_off[i] != hoff[(size_t)i]) return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: exec_out_off must be the prefix sum of exe_count (or NULL)");
-    const int64_t total = acc;
+    const int64_t total = hoff[(size_t)Q];
     if (total > out->executor_nodes_cap) return fail(c, GP_ERR_CAPACITY, "gp_pack_fifo_zones: executor_nodes_cap too small");
     if (total > 0 && !out->executor_nodes) return fail(c, GP_ERR_INVALID, "gp_pack_fifo_zones: executor_nodes is NULL");
     pitch = (pitch + 3) & ~(int64_t)3;
     GP_CUDA(c, cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
+    const bool mf = algo == GP_MINIMAL_FRAGMENTATION;
     const size_t q = (size_t)Q, T = (size_t)total, RP = (size_t)Z * (size_t)pitch;
-    size_t o = 0;
-    auto take = [&](size_t bytes) { size_t r = o; o += (bytes + 255) & ~(size_t)255; return r; };
-    const size_t o_in = take(48 * q), o_cnt = take(4 * q), o_off = take(8 * (q + 1)), o_skip = take(q), o_rexe = take(4 * RP),
-                 o_rlist = take(algo == GP_MINIMAL_FRAGMENTATION ? 8 * RP : 0), o_zone = take(4 * q), o_drv = take(4 * q),
-                 o_exe = take(4 * (T + 1)), o_avg = take(32 * q);
-    GP_CUDA(c, c->zonebuf.reserve(o));
-    char* b = c->zonebuf.as<char>();
+    int64_t *in, *d_off;
+    int32_t *cnt, *rexe, *zone, *drv, *exe;
+    uint8_t* skip;
+    int2* rlist;
+    double* avg;
+    GP_CUDA(c, stage(c->zonebuf, part(in, 6 * q), part(cnt, q), part(d_off, q + 1), part(skip, q), part(rexe, RP), part(rlist, mf ? RP : 0),
+                     part(zone, q), part(drv, q), part(exe, T + 1), part(avg, 4 * q)));
     int2* unused = nullptr;
-    gp_status s = pack_begin(c, Q, GP_TIGHTLY_PACK, mode, total, false, &unused, st);
+    s = pack_begin(c, Q, GP_TIGHTLY_PACK, mode, total, false, &unused, st);
     if (s != GP_OK) return s;
-    const int64_t* hc[6] = {a->drv_cpu_milli, a->drv_mem_bytes, a->drv_gpu, a->exe_cpu_milli, a->exe_mem_bytes, a->exe_gpu};
+    SixCols six{};
+    s = upload_apps(c, a, hoff.data(), q, st, in, cnt, d_off, six);
+    if (s != GP_OK) return s;
+    GP_CUDA(c, upload(skip, a->skip_if_no_fit, q, st));
     AppColumns cols{};
-    for (int k = 0; k < 6; ++k) {
-        if (!hc[k]) continue;
-        GP_CUDA(c, cudaMemcpyAsync(b + o_in + 8 * q * (size_t)k, hc[k], 8 * q, cudaMemcpyHostToDevice, st));
-        cols.q[k] = b + o_in + 8 * q * (size_t)k;
-    }
-    GP_CUDA(c, cudaMemcpyAsync(b + o_cnt, a->exe_count, 4 * q, cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(b + o_off, hoff.data(), 8 * (q + 1), cudaMemcpyHostToDevice, st));
-    if (a->skip_if_no_fit) GP_CUDA(c, cudaMemcpyAsync(b + o_skip, a->skip_if_no_fit, q, cudaMemcpyHostToDevice, st));
-    cols.count = (const int32_t*)(b + o_cnt); cols.group = nullptr; cols.off = (const int64_t*)(b + o_off); cols.bits = 64; cols.mem_shift = 0;
-    int* d_err = c->dev_misc.as<int>();
-    volatile int* err_host = reinterpret_cast<volatile int*>(static_cast<char*>(c->pinned_misc) + 48);
-    unsigned long long* d_stats = reinterpret_cast<unsigned long long*>(c->dev_misc.as<char>() + 8);
+    for (int k = 0; k < 6; ++k) cols.q[k] = six.p[k];
+    cols.count = cnt; cols.group = nullptr; cols.off = d_off; cols.bits = 64; cols.mem_shift = 0;
+    gp_ctx::DevStatus* ds = c->dev_status();
     PrepApp* prep = c->prep.as<PrepApp>();
     gp_prep_apps<<<(Q + kPrepThreads - 1) / kPrepThreads, kPrepThreads, 0, st>>>(
-        Q, cols, a->skip_if_no_fit ? (const uint8_t*)(b + o_skip) : nullptr, c->n_groups, total, c->snap_flags.as<SnapMeta>(), nullptr, prep, d_err, err_host);
+        Q, cols, a->skip_if_no_fit ? skip : nullptr, c->n_groups, total, c->snap_flags.as<SnapMeta>(), nullptr, prep, &ds->err, &c->status_host->err_word);
     Snapshot snap = make_snapshot(c);
     ZoneFifoIn zi{};
     const size_t N = (size_t)c->n_nodes;
     zi.sched[0] = c->sched.as<long long>(); zi.sched[1] = c->sched.as<long long>() + N; zi.sched[2] = c->sched.as<long long>() + 2 * N;
     zi.node_slot = c->node_slot.as<int32_t>();
-    zi.row_exec = (int32_t*)(b + o_rexe);
-    zi.row_list = algo == GP_MINIMAL_FRAGMENTATION ? (int2*)(b + o_rlist) : nullptr;
+    zi.row_exec = rexe;
+    zi.row_list = mf ? rlist : nullptr;
     zi.row_pitch = pitch; zi.n_apps = Q; zi.n_zones = Z;
-    double* avg = out->avg_efficiency ? (double*)(b + o_avg) : nullptr;
-    int32_t* zo = (int32_t*)(b + o_zone); int32_t* dq = (int32_t*)(b + o_drv); int32_t* eo = (int32_t*)(b + o_exe);
+    double* avg_out = out->avg_efficiency ? avg : nullptr;
     if (algo == GP_TIGHTLY_PACK) {
-        if (mode == GP_MODE_FIFO_REFERENCE) gp_pack_fifo_zones_cta<0, 1><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zo, dq, eo, avg, d_stats);
-        else gp_pack_fifo_zones_cta<0, 2><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zo, dq, eo, avg, d_stats);
+        if (mode == GP_MODE_FIFO_REFERENCE) gp_pack_fifo_zones_cta<0, 1><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zone, drv, exe, avg_out, ds->stats);
+        else gp_pack_fifo_zones_cta<0, 2><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zone, drv, exe, avg_out, ds->stats);
     } else {
-        if (mode == GP_MODE_FIFO_REFERENCE) gp_pack_fifo_zones_cta<2, 1><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zo, dq, eo, avg, d_stats);
-        else gp_pack_fifo_zones_cta<2, 2><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zo, dq, eo, avg, d_stats);
+        if (mode == GP_MODE_FIFO_REFERENCE) gp_pack_fifo_zones_cta<2, 1><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zone, drv, exe, avg_out, ds->stats);
+        else gp_pack_fifo_zones_cta<2, 2><<<1, kZoneFifoThreads, 0, st>>>(snap, prep, zi, zone, drv, exe, avg_out, ds->stats);
     }
     GP_CUDA(c, cudaGetLastError());
     c->last.kernel_launches += 2;
-    s = refresh_views(c, false, st);                   // the compact view follows the charged slots
+    s = refresh_views(c, st);                          // the compact view follows the charged slots
     if (s != GP_OK) return s;
-    GP_CUDA(c, cudaMemcpyAsync(out->zone, zo, 4 * q, cudaMemcpyDeviceToHost, st));
-    GP_CUDA(c, cudaMemcpyAsync(out->driver_node, dq, 4 * q, cudaMemcpyDeviceToHost, st));
-    if (T) GP_CUDA(c, cudaMemcpyAsync(out->executor_nodes, eo, 4 * T, cudaMemcpyDeviceToHost, st));
-    if (avg) GP_CUDA(c, cudaMemcpyAsync(out->avg_efficiency, avg, 32 * q, cudaMemcpyDeviceToHost, st));
-    GP_CUDA(c, cudaStreamSynchronize(st));
-    return decode_device_error(c, *reinterpret_cast<volatile int*>(static_cast<char*>(c->pinned_misc) + 48));
+    return zone_results_back(c, out, zone, drv, exe, avg, q, T, st);
 }
 
 gp_status gp_reserve_placements(gp_ctx* c, const gp_apps* a, const gp_results* placed, int32_t subtract, gp_reservation_table* out) {
@@ -1655,8 +1685,7 @@ gp_status gp_reserve_placements(gp_ctx* c, const gp_apps* a, const gp_results* p
     const int32_t Q = a->n_apps;
     if (out) out->n_rows = 0;
     if (Q == 0) return GP_OK;
-    if (!a->drv_cpu_milli || !a->drv_mem_bytes || !a->exe_cpu_milli || !a->exe_mem_bytes || !a->exe_count || !placed->driver_node)
-        return fail(c, GP_ERR_INVALID, "gp_reserve_placements: missing app/result arrays");
+    if (!has_requests(a) || !placed->driver_node) return fail(c, GP_ERR_INVALID, "gp_reserve_placements: missing app/result arrays");
     // host pass: offsets, rows per placed application, index validation
     std::vector<int64_t>& off = c->host_off;
     off.resize(2 * ((size_t)Q + 1));
@@ -1688,32 +1717,24 @@ gp_status gp_reserve_placements(gp_ctx* c, const gp_apps* a, const gp_results* p
     GP_CUDA(c, cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
     const size_t q = (size_t)Q, T = (size_t)(total > 0 ? total : 0), R = (size_t)rows;
-    size_t o = 0;
-    auto take = [&](size_t bytes) { size_t r = o; o += (bytes + 255) & ~(size_t)255; return r; };
-    const size_t o_in = take(48 * q), o_cnt = take(4 * q), o_off = take(8 * (q + 1)), o_roff = take(8 * (q + 1)), o_drv = take(4 * q), o_exe = take(4 * (T + 1)),
-                 o_ra = take(4 * (R + 1)), o_rs = take(4 * (R + 1)), o_rn = take(4 * (R + 1)), o_rc = take(8 * (R + 1)), o_rm = take(8 * (R + 1)), o_rg = take(8 * (R + 1));
-    GP_CUDA(c, c->zonebuf.reserve(o));
-    char* b = c->zonebuf.as<char>();
-    const int64_t* hc[6] = {a->drv_cpu_milli, a->drv_mem_bytes, a->drv_gpu, a->exe_cpu_milli, a->exe_mem_bytes, a->exe_gpu};
+    int64_t *in, *d_off, *d_roff;
+    int32_t *cnt, *drv, *exe;
+    ReserveOut ro;
+    GP_CUDA(c, stage(c->zonebuf, part(in, 6 * q), part(cnt, q), part(d_off, q + 1), part(d_roff, q + 1), part(drv, q), part(exe, T + 1),
+                     part(ro.app, R + 1), part(ro.slot, R + 1), part(ro.node, R + 1), part(ro.cpu, R + 1), part(ro.mem, R + 1), part(ro.gpu, R + 1)));
     ReserveIn ri{};
-    for (int k = 0; k < 6; ++k) {
-        if (!hc[k]) continue;
-        GP_CUDA(c, cudaMemcpyAsync(b + o_in + 8 * q * (size_t)k, hc[k], 8 * q, cudaMemcpyHostToDevice, st));
-        ri.cols.p[k] = reinterpret_cast<const int64_t*>(b + o_in + 8 * q * (size_t)k);
-    }
-    GP_CUDA(c, cudaMemcpyAsync(b + o_cnt, a->exe_count, 4 * q, cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(b + o_off, off.data(), 8 * (q + 1), cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(b + o_roff, roff, 8 * (q + 1), cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(b + o_drv, placed->driver_node, 4 * q, cudaMemcpyHostToDevice, st));
-    if (T) GP_CUDA(c, cudaMemcpyAsync(b + o_exe, placed->executor_nodes, 4 * T, cudaMemcpyHostToDevice, st));
-    ri.count = (const int32_t*)(b + o_cnt); ri.off = (const int64_t*)(b + o_off); ri.row_off = (const int64_t*)(b + o_roff);
-    ri.driver = (const int32_t*)(b + o_drv); ri.exec = (const int32_t*)(b + o_exe); ri.n_apps = Q; ri.subtract = subtract ? 1 : 0;
-    ReserveOut ro{(int32_t*)(b + o_ra), (int32_t*)(b + o_rs), (int32_t*)(b + o_rn), (long long*)(b + o_rc), (long long*)(b + o_rm), (long long*)(b + o_rg)};
+    gp_status s = upload_apps(c, a, off.data(), q, st, in, cnt, d_off, ri.cols);
+    if (s != GP_OK) return s;
+    GP_CUDA(c, upload(d_roff, roff, 8 * (q + 1), st));
+    GP_CUDA(c, upload(drv, placed->driver_node, 4 * q, st));
+    if (T) GP_CUDA(c, upload(exe, placed->executor_nodes, 4 * T, st));
+    ri.count = cnt; ri.off = d_off; ri.row_off = d_roff;
+    ri.driver = drv; ri.exec = exe; ri.n_apps = Q; ri.subtract = subtract ? 1 : 0;
     const int TH = 256;
     gp_reserve_rows<<<(unsigned)((q * 32 + TH - 1) / TH), TH, 0, st>>>(ri, ro, c->node_slot.as<int32_t>(), c->pair.as<longlong2>(), c->sgpu.as<long long>(),
                                                                         c->node_cpu.as<long long>(), c->node_mem.as<long long>(), c->node_gpu.as<long long>());
     GP_CUDA(c, cudaGetLastError());
-    if (subtract) { gp_status s = refresh_views(c, false, st); if (s != GP_OK) return s; }
+    if (subtract) { s = refresh_views(c, st); if (s != GP_OK) return s; }
     if (out && R) {
         GP_CUDA(c, cudaMemcpyAsync(out->app, ro.app, 4 * R, cudaMemcpyDeviceToHost, st));
         GP_CUDA(c, cudaMemcpyAsync(out->slot, ro.slot, 4 * R, cudaMemcpyDeviceToHost, st));
@@ -1739,20 +1760,19 @@ gp_status gp_apply_usage_delta(gp_ctx* c, int64_t n_rows, const int32_t* node, c
     GP_CUDA(c, cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
     const size_t R = (size_t)n_rows;
-    GP_CUDA(c, c->zonebuf.reserve(28 * R + 1024));
-    char* b = c->zonebuf.as<char>();
-    const size_t o_c = 0, o_m = 8 * R, o_g = 16 * R, o_n = 24 * R;
-    GP_CUDA(c, cudaMemcpyAsync(b + o_c, cpu, 8 * R, cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(b + o_m, mem, 8 * R, cudaMemcpyHostToDevice, st));
-    if (gpu) GP_CUDA(c, cudaMemcpyAsync(b + o_g, gpu, 8 * R, cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(b + o_n, node, 4 * R, cudaMemcpyHostToDevice, st));
+    long long *d_cpu, *d_mem, *d_gpu;
+    int32_t* d_node;
+    GP_CUDA(c, stage(c->zonebuf, part(d_cpu, R), part(d_mem, R), part(d_gpu, R), part(d_node, R)));
+    GP_CUDA(c, upload(d_cpu, cpu, 8 * R, st));
+    GP_CUDA(c, upload(d_mem, mem, 8 * R, st));
+    GP_CUDA(c, upload(d_gpu, gpu, 8 * R, st));
+    GP_CUDA(c, upload(d_node, node, 4 * R, st));
     const int TH = 256;
-    gp_usage_delta<<<(unsigned)((R + TH - 1) / TH), TH, 0, st>>>(n_rows, (const int32_t*)(b + o_n), (const long long*)(b + o_c), (const long long*)(b + o_m),
-                                                                  gpu ? (const long long*)(b + o_g) : nullptr, sign, c->n_nodes, c->node_slot.as<int32_t>(),
+    gp_usage_delta<<<(unsigned)((R + TH - 1) / TH), TH, 0, st>>>(n_rows, d_node, d_cpu, d_mem, gpu ? d_gpu : nullptr, sign, c->n_nodes, c->node_slot.as<int32_t>(),
                                                                   c->pair.as<longlong2>(), c->sgpu.as<long long>(), c->node_cpu.as<long long>(),
                                                                   c->node_mem.as<long long>(), c->node_gpu.as<long long>());
     GP_CUDA(c, cudaGetLastError());
-    gp_status s = refresh_views(c, sign < 0, st);
+    gp_status s = refresh_views(c, st);
     if (s != GP_OK) return s;
     GP_CUDA(c, cudaStreamSynchronize(st));
     return GP_OK;
@@ -1766,41 +1786,36 @@ static gp_status stage_availability(gp_ctx* c, const gp_usage_input* in, cudaStr
                                     long long** d_resched = nullptr) {
     const int32_t n = in->n_nodes;
     const size_t N = (size_t)n, R = (size_t)in->n_reservations;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-    const size_t o_alloc = take(24 * N), o_over = take(24 * N), o_usage = take(24 * N + 4 * N), o_avail = take(24 * N), o_sched = take(24 * N),
-                 o_resched = take(24 * N), o_rn = take(4 * R), o_rc = take(8 * R), o_rm = take(8 * R), o_rg = take(8 * R);
-    const size_t o_has = o_usage + 24 * N;      // zeroed together with the usage sums
-    GP_CUDA(c, c->usagebuf.reserve(off));
-    char* b = c->usagebuf.as<char>();
-    auto up = [&](size_t o, const void* src, size_t bytes) { return cudaMemcpyAsync(b + o, src, bytes, cudaMemcpyHostToDevice, st); };
-    GP_CUDA(c, up(o_alloc, in->alloc_cpu_milli, 8 * N));
-    GP_CUDA(c, up(o_alloc + 8 * N, in->alloc_mem_bytes, 8 * N));
-    if (in->alloc_gpu) GP_CUDA(c, up(o_alloc + 16 * N, in->alloc_gpu, 8 * N));
-    if (in->overhead_cpu_milli) GP_CUDA(c, up(o_over, in->overhead_cpu_milli, 8 * N));
-    if (in->overhead_mem_bytes) GP_CUDA(c, up(o_over + 8 * N, in->overhead_mem_bytes, 8 * N));
-    if (in->overhead_gpu) GP_CUDA(c, up(o_over + 16 * N, in->overhead_gpu, 8 * N));
-    GP_CUDA(c, cudaMemsetAsync(b + o_usage, 0, 28 * N, st));
+    long long *al, *ov, *avail, *sched, *resched, *rc, *rm, *rg;
+    char* usage_has;                            // usage sums [3][N] u64, then the has-reservation flags [N] u32: one memset
+    int32_t* rn;
+    GP_CUDA(c, stage(c->usagebuf, part(al, 3 * N), part(ov, 3 * N), part(usage_has, 28 * N), part(avail, 3 * N), part(sched, 3 * N),
+                     part(resched, 3 * N), part(rn, R), part(rc, R), part(rm, R), part(rg, R)));
+    unsigned long long* usage = reinterpret_cast<unsigned long long*>(usage_has);
+    unsigned int* has = reinterpret_cast<unsigned int*>(usage_has + 24 * N);
+    GP_CUDA(c, upload(al, in->alloc_cpu_milli, 8 * N, st));
+    GP_CUDA(c, upload(al + N, in->alloc_mem_bytes, 8 * N, st));
+    GP_CUDA(c, upload(al + 2 * N, in->alloc_gpu, 8 * N, st));
+    GP_CUDA(c, upload(ov, in->overhead_cpu_milli, 8 * N, st));
+    GP_CUDA(c, upload(ov + N, in->overhead_mem_bytes, 8 * N, st));
+    GP_CUDA(c, upload(ov + 2 * N, in->overhead_gpu, 8 * N, st));
+    GP_CUDA(c, cudaMemsetAsync(usage_has, 0, 28 * N, st));
     const int T = 256;
     if (R) {
-        GP_CUDA(c, up(o_rn, in->res_node, 4 * R));
-        GP_CUDA(c, up(o_rc, in->res_cpu_milli, 8 * R));
-        GP_CUDA(c, up(o_rm, in->res_mem_bytes, 8 * R));
-        if (in->res_gpu) GP_CUDA(c, up(o_rg, in->res_gpu, 8 * R));
-        gp_usage_scatter<<<(unsigned)((R + T - 1) / T), T, 0, st>>>((long long)R, (const int32_t*)(b + o_rn), (const long long*)(b + o_rc),
-                                                                   (const long long*)(b + o_rm), in->res_gpu ? (const long long*)(b + o_rg) : nullptr,
-                                                                   n, (unsigned long long*)(b + o_usage), d_resched ? (unsigned int*)(b + o_has) : nullptr);
+        GP_CUDA(c, upload(rn, in->res_node, 4 * R, st));
+        GP_CUDA(c, upload(rc, in->res_cpu_milli, 8 * R, st));
+        GP_CUDA(c, upload(rm, in->res_mem_bytes, 8 * R, st));
+        GP_CUDA(c, upload(rg, in->res_gpu, 8 * R, st));
+        gp_usage_scatter<<<(unsigned)((R + T - 1) / T), T, 0, st>>>((long long)R, rn, rc, rm, in->res_gpu ? rg : nullptr, n, usage,
+                                                                   d_resched ? has : nullptr);
     }
-    const long long* al = (const long long*)(b + o_alloc);
-    const long long* ov = (const long long*)(b + o_over);
     gp_availability<<<(n + T - 1) / T, T, 0, st>>>(n, al, al + N, in->alloc_gpu ? al + 2 * N : nullptr, in->overhead_cpu_milli ? ov : nullptr,
                                                    in->overhead_mem_bytes ? ov + N : nullptr, in->overhead_gpu ? ov + 2 * N : nullptr,
-                                                   (const unsigned long long*)(b + o_usage), (long long*)(b + o_avail), (long long*)(b + o_sched),
-                                                   (const unsigned int*)(b + o_has), d_resched ? (long long*)(b + o_resched) : nullptr);
-    if (d_resched) *d_resched = (long long*)(b + o_resched);
+                                                   usage, avail, sched, has, d_resched ? resched : nullptr);
+    if (d_resched) *d_resched = resched;
     GP_CUDA(c, cudaGetLastError());
-    *d_avail = (long long*)(b + o_avail);
-    *d_sched = (long long*)(b + o_sched);
+    *d_avail = avail;
+    *d_sched = sched;
     return GP_OK;
 }
 
@@ -1816,30 +1831,28 @@ static gp_status stage_sort(gp_ctx* c, const gp_sort_input* in, const long long*
         if (in->zone_id[i] < 0 || in->zone_id[i] >= in->n_zones) return fail(c, GP_ERR_INVALID, "gp_potential_nodes: zone_id out of range");
     if (in->name_rank) for (int32_t i = 0; i < n; ++i)
         if (in->name_rank[i] < 0 || in->name_rank[i] >= n) return fail(c, GP_ERR_INVALID, "gp_potential_nodes: name_rank out of range");
-    // one scratch block
     const size_t N = (size_t)n, Z = (size_t)in->n_zones;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-    const size_t o_cpu = take(8 * N), o_mem = take(8 * N), o_gpu = take(8 * N), o_keys = take(sizeof(SortKey) * N), o_sorted = take(sizeof(SortKey) * N),
-                 o_tot = take(16 * Z), o_zone = take(4 * N), o_nr = take(4 * N), o_prio = take(4 * Z), o_pos = take(4 * N), o_order = take(4 * N),
-                 o_drv = take(4 * N), o_exe = take(4 * N), o_drv2 = take(4 * N), o_exe2 = take(4 * N), o_lrd = take(4 * N),
-                 o_lre = take(4 * N), o_lk = take(sizeof(LabelKey) * N), o_lks = take(sizeof(LabelKey) * N), o_cnt = take(16),
-                 o_fc = take(N), o_fu = take(N), o_fr = take(N);
-    GP_CUDA(c, c->sortbuf.reserve(off));
-    char* b = c->sortbuf.as<char>();
-    auto up = [&](size_t o, const void* src, size_t bytes) { return cudaMemcpyAsync(b + o, src, bytes, cudaMemcpyHostToDevice, st); };
-    if (!d_cpu) { GP_CUDA(c, up(o_cpu, in->avail_cpu_milli, 8 * N)); d_cpu = (const long long*)(b + o_cpu); }
-    if (!d_mem) { GP_CUDA(c, up(o_mem, in->avail_mem_bytes, 8 * N)); d_mem = (const long long*)(b + o_mem); }
-    if (!d_gpu && in->avail_gpu) { GP_CUDA(c, up(o_gpu, in->avail_gpu, 8 * N)); d_gpu = (const long long*)(b + o_gpu); }
+    long long *cpu, *mem, *gpu;
+    SortKey *keys, *sorted;
+    LabelKey *lk, *lks;
+    unsigned long long* tot;
+    int32_t *zone, *nr, *prio, *pos, *order, *drv, *exe, *drv2, *exe2, *lrd, *lre, *cnt;
+    uint8_t *fc, *fu, *fr;
+    GP_CUDA(c, stage(c->sortbuf, part(cpu, N), part(mem, N), part(gpu, N), part(keys, N), part(sorted, N), part(tot, 2 * Z), part(zone, N),
+                     part(nr, N), part(prio, Z), part(pos, N), part(order, N), part(drv, N), part(exe, N), part(drv2, N), part(exe2, N),
+                     part(lrd, N), part(lre, N), part(lk, N), part(lks, N), part(cnt, 4), part(fc, N), part(fu, N), part(fr, N)));
+    if (!d_cpu) { GP_CUDA(c, upload(cpu, in->avail_cpu_milli, 8 * N, st)); d_cpu = cpu; }
+    if (!d_mem) { GP_CUDA(c, upload(mem, in->avail_mem_bytes, 8 * N, st)); d_mem = mem; }
+    if (!d_gpu && in->avail_gpu) { GP_CUDA(c, upload(gpu, in->avail_gpu, 8 * N, st)); d_gpu = gpu; }
     const bool zoned = in->zone_id != nullptr && in->n_zones > 1;       // one zone: priority 0 for every node, nothing to total
-    if (zoned) GP_CUDA(c, up(o_zone, in->zone_id, 4 * N));
-    if (in->name_rank) GP_CUDA(c, up(o_nr, in->name_rank, 4 * N));
-    if (in->is_driver_candidate) GP_CUDA(c, up(o_fc, in->is_driver_candidate, N));
-    if (in->unschedulable) GP_CUDA(c, up(o_fu, in->unschedulable, N));
-    if (in->ready) GP_CUDA(c, up(o_fr, in->ready, N));
-    if (in->driver_label_rank) GP_CUDA(c, up(o_lrd, in->driver_label_rank, 4 * N));
-    if (in->executor_label_rank) GP_CUDA(c, up(o_lre, in->executor_label_rank, 4 * N));
-    if (zoned) GP_CUDA(c, cudaMemsetAsync(b + o_tot, 0, 16 * Z, st));
+    if (zoned) GP_CUDA(c, upload(zone, in->zone_id, 4 * N, st));
+    GP_CUDA(c, upload(nr, in->name_rank, 4 * N, st));
+    GP_CUDA(c, upload(fc, in->is_driver_candidate, N, st));
+    GP_CUDA(c, upload(fu, in->unschedulable, N, st));
+    GP_CUDA(c, upload(fr, in->ready, N, st));
+    GP_CUDA(c, upload(lrd, in->driver_label_rank, 4 * N, st));
+    GP_CUDA(c, upload(lre, in->executor_label_rank, 4 * N, st));
+    if (zoned) GP_CUDA(c, cudaMemsetAsync(tot, 0, 16 * Z, st));
     if (!c->sort_attr_set) {
         GP_CUDA(c, cudaFuncSetAttribute(gp_sort_tiles<SortKey>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kSortTile * sizeof(SortKey))));
         c->sort_attr_set = true;
@@ -1847,35 +1860,28 @@ static gp_status stage_sort(gp_ctx* c, const gp_sort_input* in, const long long*
     const int T = 256;
     const int nb = (n + T - 1) / T;
     const int ntile = (n + kSortTile - 1) / kSortTile;
-    SortKey* keys = (SortKey*)(b + o_keys);
-    SortKey* sorted = (SortKey*)(b + o_sorted);
-    int32_t* pos = (int32_t*)(b + o_pos);
     if (zoned) {
-        gp_zone_totals<<<nb, T, 0, st>>>(n, d_cpu, d_mem, (const int32_t*)(b + o_zone), (unsigned long long*)(b + o_tot));
-        gp_zone_priority<<<(in->n_zones + T - 1) / T, T, 0, st>>>(in->n_zones, (const unsigned long long*)(b + o_tot), (int32_t*)(b + o_prio));
+        gp_zone_totals<<<nb, T, 0, st>>>(n, d_cpu, d_mem, zone, tot);
+        gp_zone_priority<<<(in->n_zones + T - 1) / T, T, 0, st>>>(in->n_zones, tot, prio);
     }
-    gp_make_keys<<<nb, T, 0, st>>>(n, d_cpu, d_mem, zoned ? (const int32_t*)(b + o_zone) : nullptr, (const int32_t*)(b + o_prio),
-                                   in->name_rank ? (const int32_t*)(b + o_nr) : nullptr, keys);
+    gp_make_keys<<<nb, T, 0, st>>>(n, d_cpu, d_mem, zoned ? zone : nullptr, prio, in->name_rank ? nr : nullptr, keys);
     gp_sort_tiles<SortKey><<<ntile, kSortThreads, kSortTile * sizeof(SortKey), st>>>(n, nullptr, keys, sorted);
     gp_rank_by_search<SortKey><<<nb, T, 0, st>>>(n, nullptr, keys, sorted, pos);
-    gp_scatter_order<<<nb, T, 0, st>>>(n, pos, (int32_t*)(b + o_order));
-    gp_split_candidates<<<1, 1024, 0, st>>>(n, (const int32_t*)(b + o_order), in->is_driver_candidate ? (const uint8_t*)(b + o_fc) : nullptr,
-                                           in->unschedulable ? (const uint8_t*)(b + o_fu) : nullptr, in->ready ? (const uint8_t*)(b + o_fr) : nullptr,
-                                           keys, d_gpu, (int32_t*)(b + o_drv), (int32_t*)(b + o_exe), (int32_t*)(b + o_cnt));
-    out->drv = (const int32_t*)(b + o_drv);
-    out->exe = (const int32_t*)(b + o_exe);
-    out->counts = (const int32_t*)(b + o_cnt);
-    auto label_sort = [&](const int32_t* cnt, const int32_t* list, size_t o_rank, size_t o_out) {
-        LabelKey* lk = (LabelKey*)(b + o_lk);
-        LabelKey* lks = (LabelKey*)(b + o_lks);
-        gp_label_keys<<<nb, T, 0, st>>>(cnt, list, (const int32_t*)(b + o_rank), lk);
-        gp_sort_tiles<LabelKey><<<ntile, kSortThreads, kSortTile * sizeof(LabelKey), st>>>(n, cnt, lk, lks);
-        gp_rank_by_search<LabelKey><<<nb, T, 0, st>>>(n, cnt, lk, lks, pos);
-        gp_label_scatter<<<nb, T, 0, st>>>(cnt, list, pos, (int32_t*)(b + o_out));
-        return (const int32_t*)(b + o_out);
+    gp_scatter_order<<<nb, T, 0, st>>>(n, pos, order);
+    gp_split_candidates<<<1, 1024, 0, st>>>(n, order, in->is_driver_candidate ? fc : nullptr, in->unschedulable ? fu : nullptr,
+                                           in->ready ? fr : nullptr, keys, d_gpu, drv, exe, cnt);
+    out->drv = drv;
+    out->exe = exe;
+    out->counts = cnt;
+    auto label_sort = [&](const int32_t* count, const int32_t* list, const int32_t* rank, int32_t* sorted_list) {
+        gp_label_keys<<<nb, T, 0, st>>>(count, list, rank, lk);
+        gp_sort_tiles<LabelKey><<<ntile, kSortThreads, kSortTile * sizeof(LabelKey), st>>>(n, count, lk, lks);
+        gp_rank_by_search<LabelKey><<<nb, T, 0, st>>>(n, count, lk, lks, pos);
+        gp_label_scatter<<<nb, T, 0, st>>>(count, list, pos, sorted_list);
+        return sorted_list;
     };
-    if (in->driver_label_rank) out->drv = label_sort(out->counts, out->drv, o_lrd, o_drv2);
-    if (in->executor_label_rank) out->exe = label_sort(out->counts + 1, out->exe, o_lre, o_exe2);
+    if (in->driver_label_rank) out->drv = label_sort(out->counts, out->drv, lrd, drv2);
+    if (in->executor_label_rank) out->exe = label_sort(out->counts + 1, out->exe, lre, exe2);
     GP_CUDA(c, cudaGetLastError());
     return GP_OK;
 }
@@ -2041,32 +2047,25 @@ gp_status gp_reschedule_executors(gp_ctx* c, const gp_reschedule* in, int32_t* n
     }
     GP_CUDA(c, cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
-    // one staging buffer: [exe 3q i64 | reserved 3N i64 | host_off (q+1) i64 | group q i32 | host_nodes H i32 | out q i32 | err i32]
     const size_t Q = (size_t)q, N = (size_t)c->n_nodes, H = (size_t)hosted;
-    const size_t o_exe = 0, o_res = o_exe + 8 * 3 * Q, o_hoff = o_res + 8 * 3 * N, o_grp = o_hoff + 8 * (Q + 1),
-                 o_hn = o_grp + 4 * Q, o_out = o_hn + 4 * (H + 1), o_err = o_out + 4 * Q, total = o_err + 8;
-    GP_CUDA(c, c->reschedbuf.reserve(total));
-    char* base = c->reschedbuf.as<char>();
-    int64_t* d_exe = reinterpret_cast<int64_t*>(base + o_exe);
-    int64_t* d_res = reinterpret_cast<int64_t*>(base + o_res);
-    int64_t* d_hoff = reinterpret_cast<int64_t*>(base + o_hoff);
-    int32_t* d_grp = reinterpret_cast<int32_t*>(base + o_grp);
-    int32_t* d_hn = reinterpret_cast<int32_t*>(base + o_hn);
-    int32_t* d_out = reinterpret_cast<int32_t*>(base + o_out);
-    int* d_err = reinterpret_cast<int*>(base + o_err);
-    GP_CUDA(c, cudaMemsetAsync(d_err, 0, 8, st));
-    GP_CUDA(c, cudaMemcpyAsync(d_exe, in->exe_cpu_milli, 8 * Q, cudaMemcpyHostToDevice, st));
-    GP_CUDA(c, cudaMemcpyAsync(d_exe + Q, in->exe_mem_bytes, 8 * Q, cudaMemcpyHostToDevice, st));
-    if (in->exe_gpu) GP_CUDA(c, cudaMemcpyAsync(d_exe + 2 * Q, in->exe_gpu, 8 * Q, cudaMemcpyHostToDevice, st));
-    if (in->group) GP_CUDA(c, cudaMemcpyAsync(d_grp, in->group, 4 * Q, cudaMemcpyHostToDevice, st));
+    int64_t *d_exe, *d_res, *d_hoff;
+    int32_t *d_grp, *d_hn, *d_out;
+    int* d_err;
+    GP_CUDA(c, stage(c->reschedbuf, part(d_exe, 3 * Q), part(d_res, 3 * N), part(d_hoff, Q + 1), part(d_grp, Q), part(d_hn, H + 1),
+                     part(d_out, Q), part(d_err, 1)));
+    GP_CUDA(c, cudaMemsetAsync(d_err, 0, sizeof(int), st));
+    GP_CUDA(c, upload(d_exe, in->exe_cpu_milli, 8 * Q, st));
+    GP_CUDA(c, upload(d_exe + Q, in->exe_mem_bytes, 8 * Q, st));
+    GP_CUDA(c, upload(d_exe + 2 * Q, in->exe_gpu, 8 * Q, st));
+    GP_CUDA(c, upload(d_grp, in->group, 4 * Q, st));
     if (has_res && N) {
-        GP_CUDA(c, cudaMemcpyAsync(d_res, in->reserved_cpu_milli, 8 * N, cudaMemcpyHostToDevice, st));
-        GP_CUDA(c, cudaMemcpyAsync(d_res + N, in->reserved_mem_bytes, 8 * N, cudaMemcpyHostToDevice, st));
-        if (in->reserved_gpu) GP_CUDA(c, cudaMemcpyAsync(d_res + 2 * N, in->reserved_gpu, 8 * N, cudaMemcpyHostToDevice, st));
+        GP_CUDA(c, upload(d_res, in->reserved_cpu_milli, 8 * N, st));
+        GP_CUDA(c, upload(d_res + N, in->reserved_mem_bytes, 8 * N, st));
+        GP_CUDA(c, upload(d_res + 2 * N, in->reserved_gpu, 8 * N, st));
     }
     if (has_host) {
-        GP_CUDA(c, cudaMemcpyAsync(d_hoff, in->host_off, 8 * (Q + 1), cudaMemcpyHostToDevice, st));
-        if (H) GP_CUDA(c, cudaMemcpyAsync(d_hn, in->host_nodes, 4 * H, cudaMemcpyHostToDevice, st));
+        GP_CUDA(c, upload(d_hoff, in->host_off, 8 * (Q + 1), st));
+        if (H) GP_CUDA(c, upload(d_hn, in->host_nodes, 4 * H, st));
     }
     ReschedIn ri{};
     ri.exe_cpu = d_exe; ri.exe_mem = d_exe + Q; ri.exe_gpu = in->exe_gpu ? d_exe + 2 * Q : nullptr;

@@ -6,6 +6,7 @@ usable, loading / context creation raises.
 from __future__ import annotations
 
 import ctypes as C
+import glob
 import os
 import shutil
 import subprocess
@@ -15,9 +16,8 @@ import numpy as np
 _PKG = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_PKG)
 LIB_PATH = os.environ.get("GANGPACK_LIB") or os.path.join(_PKG, "libgangpack.so")   # GANGPACK_LIB: experimental builds
-_SOURCES = [os.path.join(_PKG, "csrc", f) for f in ("gangpack_api.cu", "gangpack_kernels.cuh", "gangpack_fifo.cuh", "gangpack_minfrag.cuh",
-                                                    "gangpack_sort.cuh", "gangpack_tables.cuh", "gangpack_resched.cuh", "gangpack_multi.cu",
-                                                    "gangpack_zones.cuh")] + [
+# every file the library is built from: an edit to any of them makes build() recompile
+_SOURCES = sorted(glob.glob(os.path.join(_PKG, "csrc", "*.cu")) + glob.glob(os.path.join(_PKG, "csrc", "*.cuh"))) + [
     os.path.join(_ROOT, "include", "gangpack.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -60,8 +60,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
     stale = force or not os.path.exists(LIB_PATH) or any(
         os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in _SOURCES)
     if stale:
-        cmd = [_nvcc()] + NVCC_FLAGS + ["-I", os.path.join(_ROOT, "include"), "-o", LIB_PATH, _SOURCES[0],
-                                        os.path.join(_PKG, "csrc", "gangpack_multi.cu")]
+        cmd = [_nvcc()] + NVCC_FLAGS + ["-I", os.path.join(_ROOT, "include"), "-o", LIB_PATH,
+                                        os.path.join(_PKG, "csrc", "gangpack_api.cu"), os.path.join(_PKG, "csrc", "gangpack_multi.cu")]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
         subprocess.check_call(cmd)

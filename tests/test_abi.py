@@ -38,6 +38,16 @@ def test_library_exports_every_declared_symbol(native):
     assert lib.gp_abi_version() == 1
 
 
+def test_rebuild_tracks_every_source():
+    """build() recompiles when any file under csrc/ or the header is newer than the library."""
+    import k8s_spark_scheduler_b200 as g
+    csrc = os.path.join(ROOT, "k8s-spark-scheduler_b200", "csrc")
+    tracked = {os.path.abspath(s) for s in g.native._SOURCES}
+    missing = [f for f in sorted(os.listdir(csrc)) if os.path.join(csrc, f) not in tracked]
+    assert not missing, missing
+    assert os.path.join(ROOT, "include", "gangpack.h") in tracked
+
+
 def test_library_contains_sm100a_code(native):
     cuobjdump = os.path.join(os.path.dirname(native._nvcc()), "cuobjdump")   # the toolkit that built the library
     out = subprocess.check_output([cuobjdump, "-lelf", native.LIB_PATH], text=True)
